@@ -2,7 +2,7 @@
 """Headline benchmark: MLUPS of the fused D3Q19 BGK step and its HBM-roofline fraction.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                  [--n 512] [--precision f64|f32] [--storage ab|aa] [--no-e2e] [--no-cpu]
+                  [--n 512] [--precision f64|f32] [--storage ab|aa] [--no-e2e] [--no-cpu] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2]): dense lid-driven cavity 512^3, fp64, one B200.
 At N > 1 (torchrun, one rank per GPU) the domain is 1024 x 1024 x (128*N), z-slab sharded -- the
@@ -31,6 +31,11 @@ on a bounded sample of the same workload; the reference itself is a CUDA program
 size compiled in (64^3, fp32), so its kernels are reported separately under "reference_cuda": a
 patched-constant 480^3 build (baseline/_ref/variants, tools/make_reference_variants.py), with and
 without the per-kernel syncs and the thrust::reduce of its loop.
+
+--dump-outputs DIR writes what the last timed step computed -- rho, ux, uy, uz as a caller of get_fields (or of
+the oracle's fields) receives them, in the benchmark's precision -- to DIR/<name>.npy, so that two builds can be
+compared output for output on identical inputs.  Fields longer than DUMP_SAMPLE entries are replaced by the same
+seeded sample of entries on every run; at N > 1 every rank writes its own slab as <name>_rank<r>.npy.
 """
 import argparse
 import json
@@ -44,10 +49,25 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 
 BYTES_PER_LU = {"f64": 304, "f32": 152}
+DUMP_SAMPLE = 1 << 20  # entries per field and process: 32 MB for the four fp64 fields of one GPU
+
+
+def dump_outputs(out_dir, fields, rank=0, world=1):
+    """rho, ux, uy, uz to out_dir/<name>.npy; a field longer than its share of DUMP_SAMPLE is sampled at sorted
+    entries drawn with a fixed seed, which depend only on the field's length and the number of ranks"""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    keep = DUMP_SAMPLE // world
+    n = fields[0].size
+    pick = np.sort(np.random.default_rng(0).choice(n, keep, replace=False)) if n > keep else slice(None)
+    for name, a in zip(("rho", "ux", "uy", "uz"), fields):
+        assert a.dtype in (np.float32, np.float64) and a.size == n
+        np.save(out / (name if world == 1 else f"{name}_rank{rank}"), np.ascontiguousarray(a.reshape(-1)[pick]))
 
 
 def measured_peak():
@@ -207,6 +227,8 @@ def run_reference_arm(args):
     o.step(args.warmup)
     t = o.time_steps(args.steps)
     val = o.num_fluid() * args.steps / t / 1e6
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, o.fields())
     whole = n == args.n and world == 1
     sample = (f"LDC {n}^3 {args.precision}, {args.steps} steps, oracle port of ldc.cu:57-458 on {threads} host threads: "
               + ("the arm's whole workload" if whole else f"a bounded sample of the arm's workload (one {args.n}^3-sized share does not fit / is not needed: "
@@ -532,6 +554,8 @@ def run_ours(args):
         dist.all_reduce(l_)
         launches = int(l_.item())
     value = nfluid * args.steps / (ms * 1e-3) / 1e6
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, c.get_fields(), rank, world)
 
     # the dominant kernel alone (rank 0's slab), CUDA events on the launching stream
     bpl = BYTES_PER_LU[args.precision]
@@ -646,6 +670,8 @@ def main():
     ap.add_argument("--ref-n", type=int, default=0, help="cube edge of the CPU reference arm (0: the arm's own n when host memory allows)")
     ap.add_argument("--traffic-bytes", type=float, default=None,
                     help="dram__bytes_read.sum+dram__bytes_write.sum per launch from the committed ncu capture")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rho, ux, uy, uz) as DIR/<name>.npy")
     args = ap.parse_args()
     if args.storage is None:
         args.storage = "sparse_aa" if args.workload == "vessel" else "aa"

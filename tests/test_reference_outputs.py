@@ -17,8 +17,6 @@ for bit) differ by 7.6e-4.  tests/test_ldc_order_cpu.py accounts for that number
 ldc.cu's launch executes in brings the oracle to 3.4e-5 / 4.7e-5 of the real binary, which lies inside
 the envelope of the two order models; tests/test_reference_variants.py compares the library with the
 real binary at a true steady state, where the order no longer matters (5e-5, fp32 rounding)."""
-from pathlib import Path
-
 import numpy as np
 import pytest
 
@@ -136,19 +134,3 @@ def test_gpu_reproduces_reference_convergence_runs(name, rule, tol, tmp_path):
     # single-step residuals at the save iterations; noisy once below ~1e-4 (order of magnitude only)
     assert all(abs(np.log10(a) - np.log10(b)) < 1.0 for a, b in zip(log[:n], ref[:n]))
 
-
-@pytest.mark.gpu
-def test_live_reference_binary_if_present(tmp_path):
-    """when oracle/_ref was built (authoring container) run the reference itself, here, now"""
-    import subprocess
-
-    exe = Path(__file__).resolve().parents[1] / "oracle" / "_ref" / "pos_ref"
-    if not exe.exists():
-        pytest.skip("oracle/_ref not built")
-    (tmp_path / "out").mkdir()
-    r = subprocess.run([str(exe)], cwd=tmp_path, capture_output=True, text=True, timeout=600)
-    assert "TOTAL RUNNING TIME" in r.stdout
-    last = max(tmp_path.glob("out/pos_*.vtk"), key=lambda p: int(p.stem.split("_")[1]))
-    assert int(last.stem.split("_")[1]) == int(GOLD["pos_last_iter"])
-    body = np.array(last.read_text().split("\n")[9].split(), dtype=np.float32).reshape(62, 60, 62, 3)
-    compare("pos", body, 1e-6)
