@@ -274,7 +274,9 @@ int lbm_last_velsum(lbm_handle h, double *value);
  *                   as exported) at peer_halo_c0 = the neighbour's halo-plane offset facing this slab;
  *                   peer_face_c0 = offset of the neighbour's outermost OWNED plane on that side, which
  *                   the odd step of the in-place (AA) storage pushes into.  With in-place storage the
- *                   peer stores are the only transport: attach before stepping a slab. */
+ *                   peer stores are the only transport: attach before stepping a slab.  Null buffers
+ *                   detach.  While either side of the slab holds a mailbox (lbm_mail_attach or
+ *                   lbm_mail_stage), this returns LBM_ERR_STATE: detach it first. */
 typedef struct {
     unsigned char bytes[64];
 } lbm_ipc_handle;
@@ -311,7 +313,8 @@ int lbm_sync_attach(lbm_handle h, int32_t side, void *peer_sync);
  * the face launches read the entering populations from the own mailbox (base-pointer redirection, the kernel does
  * not know) and store the leaving ones into the neighbour's.  Both slabs of a face switch together, between two
  * steps; checkpoints and lbm_debug_get_populations see the complete population buffer (the mailbox is drained and
- * re-filled around them).  LBM_STORE_DENSE_AA only. */
+ * re-filled around them).  LBM_STORE_DENSE_AA only.  A null peer_mail detaches either kind of mailbox; while either side
+ * of the slab holds mapped buffers (lbm_p2p_attach) or a staged mailbox, this returns LBM_ERR_STATE: detach it first. */
 int lbm_mail_export(lbm_handle h, int32_t side, lbm_ipc_handle *handle, void **ptr, int64_t *byte_offset, int64_t *stride,
                     int64_t *guard);
 int lbm_mail_attach(lbm_handle h, int32_t side, void *peer_mail);
@@ -320,7 +323,8 @@ int lbm_mail_attach(lbm_handle h, int32_t side, void *peer_mail);
  * store the leaving populations into the local send part, lbm_halo_buffers(side) returns the send / receive part
  * of the current step (5 planes each), the caller moves send -> the neighbour's receive between lbm_step_begin and
  * lbm_step_end (ordered on lbm_stream), and lbm_step_end merges what arrived into the mailbox.  Steps are driven
- * with lbm_step_begin / lbm_step_interior / lbm_step_end as for the two-buffer storage. */
+ * with lbm_step_begin / lbm_step_interior / lbm_step_end as for the two-buffer storage; lbm_mail_attach(side, NULL) ends
+ * it.  While either side of the slab holds mapped buffers or a mapped mailbox, this returns LBM_ERR_STATE: detach it. */
 int lbm_mail_stage(lbm_handle h, int32_t side);
 
 /* ---- several z-slabs driven from ONE process: the multi-GPU form of the reference's main() ----

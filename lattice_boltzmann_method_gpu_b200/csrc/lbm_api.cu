@@ -73,7 +73,6 @@ struct SolverBase {
     virtual double *acc_slot(int k) = 0;
     virtual int write_global(int t, const int32_t *index_global, const void *rho, const void *ux, const void *uy,
                              const void *uz, int64_t nlattice) = 0;
-    bool lo_halo_b = false, hi_halo_b = false;
     virtual int residual(int kind, double *v) = 0;
     virtual int get_geo(int32_t *g) = 0;
     virtual int get_index(int32_t *g) = 0;
@@ -137,7 +136,6 @@ struct Solver final : SolverBase {
     T *d_fa = nullptr, *d_fb = nullptr, *d_cur = nullptr, *d_nxt = nullptr;
     T *d_rho = nullptr, *d_ux = nullptr, *d_uy = nullptr, *d_uz = nullptr;
     T *d_plane_in = nullptr, *d_plane_out = nullptr;
-    T *d_send[2] = {nullptr, nullptr}, *d_recv[2] = {nullptr, nullptr};
     double *d_acc = nullptr;      // [ACC_SLOTS] reduction slots
     long long *d_cnt = nullptr;   // small device counters
     static constexpr int ACC_SLOTS = 64;
@@ -153,21 +151,32 @@ struct Solver final : SolverBase {
     cudaEvent_t ev_gathered[2] = {nullptr, nullptr}, ev_copied[2] = {nullptr, nullptr};
     long long pend_i0 = 0, pend_i1 = 0;
     bool interior_pending = false;
-    // fused peer-to-peer halo exchange (per side: neighbour's two buffers, q stride, halo offset)
-    T *peer_buf[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};
-    long long peer_qs[2] = {0, 0}, peer_c0[2] = {0, 0}, peer_own[2] = {0, 0};
-    // mailboxes of the dense in-place storage (StepParams::mail): own ones per side, the neighbours' as mapped here
-    T *d_mail[2] = {nullptr, nullptr}, *peer_mail[2] = {nullptr, nullptr};
-    long long mail_ms = 0, mail_G = 0;
-    bool mail_live[2] = {false, false};  // the mailbox, not the population buffer, holds the current values of its slots
-    T *d_stage_out[2] = {nullptr, nullptr}, *d_stage_in[2] = {nullptr, nullptr};  // staged mailboxes (lbm_mail_stage)
-    bool mail_staged[2] = {false, false};
-    // neighbour ordering of slab steps: flags in peer memory (other process) or events (same process)
+    // How the populations crossing one z face reach the neighbour (include/lbm_b200.h, "z-slab halo exchange" on):
+    //   PACKED          the step packs them into `send` and unpacks the neighbour's from `recv`; the caller moves the bytes
+    //   PEER_BUFFERS    the face launches store into the neighbour's population buffers (lbm_p2p_attach)
+    //   MAILBOX         ... into the neighbour's mailbox, and read the entering ones from `mail` (lbm_mail_attach)
+    //   STAGED_MAILBOX  ... into `stage_out`; the caller moves it to the neighbour's `stage_in`, which lbm_step_end
+    //                   merges into `mail` (lbm_mail_stage)
+    // The kinds change only in the "slab faces" section (relink, unlink_*); a step asks the face what to do there too.
+    enum class Link { PACKED, PEER_BUFFERS, MAILBOX, STAGED_MAILBOX };
+    struct Face {
+        Link kind = Link::PACKED;
+        T *send = nullptr, *recv = nullptr;       // pack / unpack buffers, allocated by initialize for every kind
+        T *peer_buf[2] = {nullptr, nullptr};      // PEER_BUFFERS: the neighbour's two buffers in export order,
+        long long peer_qs = 0, peer_c0 = 0, peer_own = 0;  // their q stride, halo-plane and outermost-owned-plane offsets
+        T *mail = nullptr;                        // own mailbox (lbm_mail_export, 10 planes), kept when the kind changes
+        T *peer_mail = nullptr;                   // MAILBOX: the neighbour's mailbox as mapped here; STAGED: stage_out
+        bool mail_live = false;  // the mailbox, not the population buffer, holds the current values of its slots
+        T *stage_out = nullptr, *stage_in = nullptr;  // STAGED_MAILBOX: send / receive parts, A and B halves each
+        unsigned long long *peer_sync = nullptr;  // ordering: where this slab reports its progress (other process), or
+        SolverBase *inproc_nb = nullptr;          // the neighbour whose face events it waits for (same process)
+        bool mailbox() const { return kind == Link::MAILBOX || kind == Link::STAGED_MAILBOX; }
+    };
+    Face face[2];                                       // [0] low-z side, [1] high-z side
+    long long mail_ms = 0, mail_G = 0;                  // mailbox plane stride and guard (StepParams::mail)
     unsigned long long *d_sync = nullptr;               // [0] low neighbour's progress, [1] high neighbour's, [2] timeout
-    unsigned long long *peer_sync[2] = {nullptr, nullptr};  // where this slab reports its own progress, per side
     int64_t sync_base = 0;                              // step count at which the progress counters were zero
     cudaEvent_t ev_face[2] = {nullptr, nullptr};        // recorded after the face launches of even / odd steps
-    SolverBase *inproc_nb[2] = {nullptr, nullptr};
     // sparse storage (reference compact order + run segments)
     bool sparse = false;
     long long n_lo_stored = 0, stored_box = 0;   // stored nodes of the low halo plane / of the whole state box
@@ -197,10 +206,10 @@ struct Solver final : SolverBase {
         };
         fr(d_flag), fr(d_label_ext), fr(d_label), fr(d_index), fr(d_scratch), fr(d_node), fr(d_seg), fr(d_label8);
         fr(d_fa), fr(d_fb == d_fa ? nullptr : d_fb), fr(d_rho), fr(d_ux), fr(d_uy), fr(d_uz), fr(d_plane_in), fr(d_plane_out);
-        fr(d_send[0]), fr(d_send[1]), fr(d_recv[0]), fr(d_recv[1]), fr(d_acc), fr(d_cnt);
+        fr(d_acc), fr(d_cnt);
         fr(d_sid), fr(d_cmeta), fr(d_rec_links), fr(d_bcslot), fr(d_bclinks);
         fr(d_stage), fr(d_wall), fr(d_wallc), fr(d_cart), fr(d_chunk_off), fr(d_nodec), fr(d_labelc), fr(d_rec), fr(d_chunk_cnt), fr(d_plane_seg);
-        fr(d_mail[0]), fr(d_mail[1]), fr(d_stage_out[0]), fr(d_stage_out[1]), fr(d_stage_in[0]), fr(d_stage_in[1]);
+        for (Face &f : face) fr(f.send), fr(f.recv), fr(f.mail), fr(f.stage_out), fr(f.stage_in);
         fr(d_sync), fr(d_chk_shadow[0]), fr(d_chk_shadow[1]), fr(d_chk_count), fr(d_pulse), fr(d_barrier);
         if (ev0) cudaEventDestroy(ev0);
         if (ev1) cudaEventDestroy(ev1);
@@ -244,13 +253,12 @@ struct Solver final : SolverBase {
     void release_geometry_sized() {
         if (d_fb == d_fa) d_fb = nullptr;
         dfree(&d_fa), dfree(&d_fb), dfree(&d_rho), dfree(&d_ux), dfree(&d_uy), dfree(&d_uz);
-        for (int sd = 0; sd < 2; sd++) dfree(&d_send[sd]), dfree(&d_recv[sd]);
         dfree(&d_cart), dfree(&d_nodec), dfree(&d_wallc), dfree(&d_labelc), dfree(&d_rec), dfree(&d_chunk_cnt);
         dfree(&d_cmeta), dfree(&d_rec_links), dfree(&d_bcslot), dfree(&d_bclinks);
         dfree(&d_chunk_off), dfree(&d_plane_seg);
         if (d_stage) cudaFree(d_stage), d_stage = nullptr, stage_elems = 0;
         d_cur = d_nxt = nullptr;
-        for (int sd = 0; sd < 2; sd++) peer_buf[sd][0] = peer_buf[sd][1] = nullptr;
+        unlink_geometry_sized();
     }
 
     int setup() {
@@ -262,7 +270,6 @@ struct Solver final : SolverBase {
         fluid_label = d.case_rule == LBM_CASE_LDC ? 3 : 4;
         own_z0 = d.z_begin, own_z1 = d.z_end;
         lo_halo = own_z0 > 0, hi_halo = own_z1 < d.nz;
-        lo_halo_b = lo_halo, hi_halo_b = hi_halo;
         const int px = ((d.nx + 31) / 32) * 32;
         box.nx = d.nx, box.ny = d.ny, box.nz = d.nz, box.px = px, box.plane = (long long)px * d.ny;
         box.z0 = own_z0 - (lo_halo ? 1 : 0), box.z1 = own_z1 + (hi_halo ? 1 : 0);
@@ -552,9 +559,8 @@ struct Solver final : SolverBase {
             if (dalloc(&d_rho, (size_t)cells) || dalloc(&d_ux, (size_t)cells) || dalloc(&d_uy, (size_t)cells) ||
                 dalloc(&d_uz, (size_t)cells))
                 return LBM_ERR_NOMEM;
-            for (int s = 0; s < 2; s++)
-                if (dalloc(&d_send[s], (size_t)box.plane * 5) || dalloc(&d_recv[s], (size_t)box.plane * 5))
-                    return LBM_ERR_NOMEM;
+            for (Face &f : face)
+                if (dalloc(&f.send, (size_t)box.plane * 5) || dalloc(&f.recv, (size_t)box.plane * 5)) return LBM_ERR_NOMEM;
         }
         InitParams<T> ip{};
         ip.fa = d_fa, ip.fb = d_fb, ip.aa = aa ? 1 : 0, ip.qstride = qstride, ip.label = d_label;
@@ -568,17 +574,8 @@ struct Solver final : SolverBase {
         d_cur = d_fa, d_nxt = d_fb;
         steps = 0;
         have_init = true, have_moments = false, in_step = false;
-        detach_neighbours();
+        unlink_initialized();
         return 0;
-    }
-    // a freshly initialised slab has no ordering with its neighbours yet (lbm_sync_attach / the group wire it)
-    void detach_neighbours() {
-        peer_sync[0] = peer_sync[1] = nullptr;
-        inproc_nb[0] = inproc_nb[1] = nullptr;
-        peer_mail[0] = peer_mail[1] = nullptr;
-        mail_live[0] = mail_live[1] = false;
-        mail_staged[0] = mail_staged[1] = false;
-        sync_base = 0;
     }
 
     long long count_plane(int zl) {
@@ -709,7 +706,7 @@ struct Solver final : SolverBase {
                 return LBM_ERR_NOMEM;
             for (int sd = 0; sd < 2; sd++) {
                 const size_t nb = (size_t)std::max(face_n[sd], halo_n[sd]) * 5;
-                if (dalloc(&d_send[sd], nb) || dalloc(&d_recv[sd], nb)) return LBM_ERR_NOMEM;
+                if (dalloc(&face[sd].send, nb) || dalloc(&face[sd].recv, nb)) return LBM_ERR_NOMEM;
             }
         }
         InitParams<T> ip{};
@@ -724,7 +721,7 @@ struct Solver final : SolverBase {
         d_cur = d_fa, d_nxt = d_fb;
         steps = 0;
         have_init = true, have_moments = false, in_step = false;
-        detach_neighbours();
+        unlink_initialized();
         return 0;
     }
 
@@ -776,25 +773,9 @@ struct Solver final : SolverBase {
     int launch_range(long long c0, long long c1, bool moments, bool resid, double *acc, int face_sides = 0) {
         if (c1 <= c0) return 0;
         StepParams<T> p = make_params(c0, c1, acc);
-        // face_sides bit 0: this range is the lowest owned plane, bit 1: the highest -> push to attached peers
-        const int which = d_nxt == d_fa ? 0 : 1;
-        for (int sd = 0; sd < 2; sd++) {
-            if (!(face_sides & (1 << sd)) || !peer_mail[sd]) continue;
-            // the neighbour's mailbox: part A (its halo replica) on even steps, part B (its owned face plane) on odd ones
-            T *dst = peer_mail[sd] + (p.parity ? 5 * mail_ms : 0);
-            if (sd == 1) p.peer_up = dst, p.peer_up_qs = mail_ms, p.peer_up_c0 = mail_G, p.peer_up_own = mail_G;
-            else p.peer_dn = dst, p.peer_dn_qs = mail_ms, p.peer_dn_c0 = mail_G, p.peer_dn_own = mail_G;
-            p.peer_mail = 1, p.face_c0 = c0;
-            p.mail[sd] = d_mail[sd], p.mail_ms = mail_ms, p.mail_G = mail_G;
-        }
-        if ((face_sides & 2) && peer_buf[1][which]) {
-            p.peer_up = peer_buf[1][which], p.peer_up_qs = peer_qs[1], p.peer_up_c0 = peer_c0[1], p.peer_up_own = peer_own[1];
-            p.face_c0 = sparse ? face_id0[1] : c0;
-        }
-        if ((face_sides & 1) && peer_buf[0][which]) {
-            p.peer_dn = peer_buf[0][which], p.peer_dn_qs = peer_qs[0], p.peer_dn_c0 = peer_c0[0], p.peer_dn_own = peer_own[0];
-            p.face_c0 = sparse ? face_id0[0] : c0;
-        }
+        // face_sides bit 0: this range is the lowest owned plane, bit 1: the highest
+        for (int sd = 0; sd < 2; sd++)
+            if (face_sides & (1 << sd)) link_params(p, sd, c0);
         if (sparse) {
             SparseParams<T> sp{};
             sp.base = p, sp.rec = d_rec, sp.nodec = d_nodec, sp.wallc = d_wallc;
@@ -926,7 +907,7 @@ struct Solver final : SolverBase {
         if (in_step) FAIL(LBM_ERR_STATE, "lbm_step_begin called twice");
         CK(cudaSetDevice(d.device));
         const bool mom = flags & LBM_STEP_MOMENTS, res = flags & LBM_STEP_VELSUM;
-        if (in_place() && ((lo_halo && !peer_buf[0][0] && !peer_mail[0]) || (hi_halo && !peer_buf[1][0] && !peer_mail[1])))
+        if (in_place() && ((lo_halo && !fused(0)) || (hi_halo && !fused(1))))
             FAIL(LBM_ERR_STATE, "in-place storage exchanges slab faces by peer stores only: call lbm_p2p_attach first");
         step_flags = flags;
         step_acc = acc ? acc : d_acc, step_nosync = acc != nullptr;
@@ -934,39 +915,31 @@ struct Solver final : SolverBase {
         // a slab may touch the planes it shares with a neighbour only after that neighbour finished the
         // face launches of the previous step (flags across processes, events inside one)
         const unsigned long long done = (unsigned long long)(steps - sync_base);
-        if (peer_sync[0] || peer_sync[1]) {
-            CK(launch_slab_wait(d_sync, peer_sync[0] ? done : 0ull, peer_sync[1] ? done : 0ull, SYNC_TIMEOUT_NS, st));
+        if (face[0].peer_sync || face[1].peer_sync) {
+            CK(launch_slab_wait(d_sync, face[0].peer_sync ? done : 0ull, face[1].peer_sync ? done : 0ull, SYNC_TIMEOUT_NS, st));
             launches++;
         }
-        for (int sd = 0; sd < 2; sd++)
-            if (inproc_nb[sd]) CK(cudaStreamWaitEvent(st, inproc_nb[sd]->face_event((int)((steps + 1) & 1)), 0));
+        for (const Face &f : face)
+            if (f.inproc_nb) CK(cudaStreamWaitEvent(st, f.inproc_nb->face_event((int)((steps + 1) & 1)), 0));
         int r;
         const int zt = own_z1 - 1, zb = own_z0;
         long long i0 = plane_c(own_z0), i1 = plane_c(own_z1);
         if (hi_halo) {
             const int sides = 2 | ((lo_halo && zb == zt) ? 1 : 0);
             if ((r = launch_range(plane_c(zt), plane_c(zt + 1), mom, res, step_acc, sides))) return r;
-            if (!fused(1)) {
-                if (sparse) CK(launch_halo_pack_sparse<T>(d_nxt, qstride, face_id0[1], face_n[1], 1, d_send[1], face_n[1], st));
-                else CK(launch_halo_pack<T>(d_nxt, qstride, box, zt - box.z0, 1, d_send[1], st));
-                launches++;
-            }
+            if ((r = after_face_launch(1))) return r;
             i1 = plane_c(zt);
         }
         if (lo_halo && !(hi_halo && zb == zt)) {
             if ((r = launch_range(plane_c(zb), plane_c(zb + 1), mom, res, step_acc, 1))) return r;
             i0 = plane_c(zb + 1);
         }
-        if (lo_halo && !fused(0)) {
-            if (sparse) CK(launch_halo_pack_sparse<T>(d_nxt, qstride, face_id0[0], face_n[0], 0, d_send[0], face_n[0], st));
-            else CK(launch_halo_pack<T>(d_nxt, qstride, box, zb - box.z0, 0, d_send[0], st));
+        if (lo_halo && (r = after_face_launch(0))) return r;
+        if (face[0].peer_sync || face[1].peer_sync) {
+            CK(launch_slab_signal(face[0].peer_sync, face[1].peer_sync, done + 1ull, st));
             launches++;
         }
-        if (peer_sync[0] || peer_sync[1]) {
-            CK(launch_slab_signal(peer_sync[0], peer_sync[1], done + 1ull, st));
-            launches++;
-        }
-        if (inproc_nb[0] || inproc_nb[1]) CK(cudaEventRecord(ev_face[steps & 1], st));
+        if (face[0].inproc_nb || face[1].inproc_nb) CK(cudaEventRecord(ev_face[steps & 1], st));
         pend_i0 = i0, pend_i1 = i1, interior_pending = true;
         in_step = true;
         return 0;
@@ -987,25 +960,10 @@ struct Solver final : SolverBase {
             int r = step_interior();
             if (r) return r;
         }
-        if (lo_halo && !fused(0)) {
-            if (sparse) CK(launch_halo_unpack_sparse<T>(d_nxt, qstride, d_labelc, fluid_label, halo_id0[0], halo_n[0], 0, d_recv[0], halo_n[0], st));
-            else CK(launch_halo_unpack<T>(d_nxt, qstride, d_label8, fluid_label, box, 0, 0, d_recv[0], st));
-            launches++;
+        for (int sd = 0; sd < 2; sd++) {
+            int r = has_nb(sd) ? at_step_end(sd) : 0;
+            if (r) return r;
         }
-        if (hi_halo && !fused(1)) {
-            if (sparse) CK(launch_halo_unpack_sparse<T>(d_nxt, qstride, d_labelc, fluid_label, halo_id0[1], halo_n[1], 1, d_recv[1], halo_n[1], st));
-            else CK(launch_halo_unpack<T>(d_nxt, qstride, d_label8, fluid_label, box, box.z1 - box.z0 - 1, 1, d_recv[1], st));
-            launches++;
-        }
-        for (int sd = 0; sd < 2; sd++)
-            if ((sd == 0 ? lo_halo : hi_halo) && mail_staged[sd]) {
-                // take over what the neighbour stored (the transfer into the receive part is complete on this stream),
-                // and give the part that was sent its "nothing written" pattern back
-                const size_t off = (steps & 1) ? (size_t)mail_ms * 5 : 0;
-                CK(launch_mail_merge<T>(d_mail[sd] + off, d_stage_in[sd] + off, mail_ms * 5, st));
-                CK(cudaMemsetAsync(d_stage_out[sd] + off, 0xFF, (size_t)mail_ms * 5 * sizeof(T), st));
-                launches++;
-            }
         if ((step_flags & LBM_STEP_VELSUM) && !step_nosync) {
             CK(cudaMemcpyAsync(&last_S, d_acc, sizeof(double), cudaMemcpyDeviceToHost, st));
             CK(cudaStreamSynchronize(st));
@@ -1036,7 +994,7 @@ struct Solver final : SolverBase {
         return check_sync_error();
     }
     int check_sync_error() {
-        if (!peer_sync[0] && !peer_sync[1]) return 0;
+        if (!face[0].peer_sync && !face[1].peer_sync) return 0;
         unsigned long long flag = 0;
         CK(cudaMemcpyAsync(&flag, d_sync + 2, sizeof flag, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
@@ -1044,15 +1002,15 @@ struct Solver final : SolverBase {
         return 0;
     }
     cudaEvent_t face_event(int k) override { return ev_face[k & 1]; }
-    void set_inproc_neighbour(int side, SolverBase *nb) override { inproc_nb[side] = nb; }
+    void set_inproc_neighbour(int side, SolverBase *nb) override { face[side].inproc_nb = nb; }
     // lbm_slab_step: n steps of this slab, neighbours ordered on the device, nothing but launches on the host
     int slab_steps(int n, int flags_last, double *S_out, float *ms) override {
         if (!have_init) FAIL(LBM_ERR_STATE, "step before initialize");
         if (n < 0) FAIL(LBM_ERR_ARG, "negative step count");
         for (int sd = 0; sd < 2; sd++) {
-            if (!(sd == 0 ? lo_halo : hi_halo)) continue;
-            if (!peer_buf[sd][0] && !peer_mail[sd]) FAIL(LBM_ERR_STATE, "lbm_slab_step needs the fused peer-store exchange: lbm_p2p_attach side %d first", sd);
-            if (!peer_sync[sd] && !inproc_nb[sd])
+            if (!has_nb(sd)) continue;
+            if (!fused(sd)) FAIL(LBM_ERR_STATE, "lbm_slab_step needs the fused peer-store exchange: lbm_p2p_attach side %d first", sd);
+            if (!face[sd].peer_sync && !face[sd].inproc_nb)
                 FAIL(LBM_ERR_STATE, "lbm_slab_step: no ordering with the neighbour on side %d (lbm_sync_attach)", sd);
         }
         CK(cudaSetDevice(d.device));
@@ -1080,80 +1038,165 @@ struct Solver final : SolverBase {
         }
         return check_sync_error();
     }
-    bool fused(int sd) const { return peer_buf[sd][0] != nullptr || peer_mail[sd] != nullptr; }
-    long long halo_cell0(int side) const { return side == 0 ? 0 : (long long)(box.z1 - box.z0 - 1) * box.plane; }
-    long long face_cell0(int side) const { return side == 0 ? plane_c(own_z0) : plane_c(own_z1 - 1); }
-    // move the slots of the entering directions between the population buffer and a side's mailbox
-    int mail_move(int side, int dir) {
-        CK(launch_mail_copy<T>(d_fa, qstride, d_mail[side], mail_ms, mail_G, face_cell0(side), halo_cell0(side), box.plane, side, dir, st));
+    // ------------------------------------------------------------ slab faces (Face, Link)
+    bool has_nb(int sd) const { return sd == 0 ? lo_halo : hi_halo; }
+    // the step kernels store the leaving populations of this face themselves: no pack, no unpack
+    bool fused(int sd) const { return face[sd].kind != Link::PACKED; }
+    // the StepParams peer fields of a launch that covers side sd's face plane (c0: the launch's first cell)
+    void link_params(StepParams<T> &p, int sd, long long c0) const {
+        const Face &f = face[sd];
+        T *peer = nullptr;
+        long long qs = 0, pc0 = 0, own = 0;
+        switch (f.kind) {
+        case Link::PACKED:
+            return;
+        case Link::PEER_BUFFERS:
+            peer = f.peer_buf[d_nxt == d_fa ? 0 : 1], qs = f.peer_qs, pc0 = f.peer_c0, own = f.peer_own;
+            p.face_c0 = sparse ? face_id0[sd] : c0;
+            break;
+        case Link::MAILBOX:
+        case Link::STAGED_MAILBOX:
+            // the neighbour's mailbox: part A (its halo replica) on even steps, part B (its owned face plane) on odd ones
+            peer = f.peer_mail + (p.parity ? 5 * mail_ms : 0), qs = mail_ms, pc0 = own = mail_G;
+            p.peer_mail = 1, p.face_c0 = c0;
+            p.mail[sd] = f.mail, p.mail_ms = mail_ms, p.mail_G = mail_G;
+            break;
+        }
+        if (sd == 1) p.peer_up = peer, p.peer_up_qs = qs, p.peer_up_c0 = pc0, p.peer_up_own = own;
+        else p.peer_dn = peer, p.peer_dn_qs = qs, p.peer_dn_c0 = pc0, p.peer_dn_own = own;
+    }
+    // queued right after the launch of side sd's face plane: the pack of a PACKED face
+    int after_face_launch(int sd) {
+        const Face &f = face[sd];
+        if (f.kind != Link::PACKED) return 0;
+        if (sparse) CK(launch_halo_pack_sparse<T>(d_nxt, qstride, face_id0[sd], face_n[sd], sd, f.send, face_n[sd], st));
+        else CK(launch_halo_pack<T>(d_nxt, qstride, box, (sd == 0 ? own_z0 : own_z1 - 1) - box.z0, sd, f.send, st));
         launches++;
         return 0;
     }
-    // make the population buffer complete again (before it is read as a whole or the neighbours change)
-    int mail_drain() {
-        for (int sd = 0; sd < 2; sd++)
-            if (mail_live[sd]) {
-                int r = mail_move(sd, 1);
-                if (r) return r;
-                mail_live[sd] = false;
-            }
+    // queued by lbm_step_end, after the caller's transfers into the receive buffers
+    int at_step_end(int sd) {
+        const Face &f = face[sd];
+        if (f.kind == Link::PACKED) {
+            if (sparse) CK(launch_halo_unpack_sparse<T>(d_nxt, qstride, d_labelc, fluid_label, halo_id0[sd], halo_n[sd], sd, f.recv, halo_n[sd], st));
+            else CK(launch_halo_unpack<T>(d_nxt, qstride, d_label8, fluid_label, box, sd == 0 ? 0 : box.z1 - box.z0 - 1, sd, f.recv, st));
+            launches++;
+        } else if (f.kind == Link::STAGED_MAILBOX) {
+            // take over what the neighbour stored (the transfer into the receive part is complete on this stream),
+            // and give the part that was sent its "nothing written" pattern back
+            const size_t off = (steps & 1) ? (size_t)mail_ms * 5 : 0;
+            CK(launch_mail_merge<T>(f.mail + off, f.stage_in + off, mail_ms * 5, st));
+            CK(cudaMemsetAsync(f.stage_out + off, 0xFF, (size_t)mail_ms * 5 * sizeof(T), st));
+            launches++;
+        }
         return 0;
     }
-    int mail_refill() {
-        for (int sd = 0; sd < 2; sd++)
-            if (peer_mail[sd] && !mail_live[sd]) {
-                int r = mail_move(sd, 0);
-                if (r) return r;
-                mail_live[sd] = true;
-            }
+    // Every attach and detach of the C ABI, between two steps; the caller fills in the new kind's peer pointers.
+    // Both faces of a slab hold the same fused kind: a one-plane slab's launch covers both with one StepParams, whose
+    // peer_mail flag tells the kernel how to address both peers.  So changing the kind needs a detach first.
+    int relink(int sd, Link kind) {
+        static const char *const names[] = {"packed", "peer-buffer", "mailbox", "staged-mailbox"};
+        for (int s = 0; s < 2; s++)
+            if (kind != Link::PACKED && face[s].kind != Link::PACKED && face[s].kind != kind)
+                FAIL(LBM_ERR_STATE, "side %d holds a %s link: detach it before attaching a %s link to side %d", s,
+                     names[(int)face[s].kind], names[(int)kind], sd);
+        CK(cudaSetDevice(d.device));
+        CK(cudaStreamSynchronize(st));
+        int r = mail_place(sd, kind == Link::MAILBOX || kind == Link::STAGED_MAILBOX);
+        if (r) return r;
+        CK(cudaStreamSynchronize(st));
+        Face &f = face[sd];
+        f.kind = kind;
+        f.peer_buf[0] = f.peer_buf[1] = f.peer_mail = nullptr;
+        f.peer_qs = f.peer_c0 = f.peer_own = 0;
         return 0;
+    }
+    // Where the current values of side sd's mailbox slots (the entering directions) are: in its mailbox (live) or in
+    // the population buffer.  The population buffer is made whole before it is read as a whole (checkpoints,
+    // lbm_debug_get_populations) and handed back to the mailboxes afterwards: mail_place_all(false / true).
+    int mail_place(int sd, bool live) {
+        Face &f = face[sd];
+        if (f.mail_live == live) return 0;
+        const long long halo_c0 = sd == 0 ? 0 : (long long)(box.z1 - box.z0 - 1) * box.plane;
+        const long long face_c0 = sd == 0 ? plane_c(own_z0) : plane_c(own_z1 - 1);
+        CK(launch_mail_copy<T>(d_fa, qstride, f.mail, mail_ms, mail_G, face_c0, halo_c0, box.plane, sd, live ? 0 : 1, st));
+        launches++;
+        f.mail_live = live;
+        return 0;
+    }
+    int mail_place_all(bool live) {
+        for (int sd = 0; sd < 2; sd++) {
+            int r = mail_place(sd, live && face[sd].mailbox());
+            if (r) return r;
+        }
+        return 0;
+    }
+    // initialize: the population buffer was just written whole, so mailbox links end without moving slots back;
+    // mapped peer buffers stay, and the ordering with the neighbours is wired again (lbm_sync_attach / the group)
+    void unlink_initialized() {
+        for (Face &f : face) {
+            if (f.mailbox()) f.kind = Link::PACKED, f.peer_mail = nullptr;
+            f.mail_live = false, f.peer_sync = nullptr, f.inproc_nb = nullptr;
+        }
+        sync_base = 0;
+    }
+    // geo_pre of an initialised sparse slab: the pack buffers and the neighbours' buffers fit the old geometry
+    void unlink_geometry_sized() {
+        for (Face &f : face) {
+            dfree(&f.send), dfree(&f.recv);
+            if (f.kind == Link::PEER_BUFFERS) f.kind = Link::PACKED, f.peer_buf[0] = f.peer_buf[1] = nullptr;
+        }
     }
     int mail_export(int side, lbm_ipc_handle *h, void **ptr, int64_t *boff, int64_t *ms, int64_t *guard) override {
         if (side < 0 || side > 1) FAIL(LBM_ERR_ARG, "side must be 0 or 1");
         if (!have_init) FAIL(LBM_ERR_STATE, "mail_export before initialize");
         if (d.storage != LBM_STORE_DENSE_AA) FAIL(LBM_ERR_STATE, "mailboxes exist for the dense in-place storage only");
-        if (!(side == 0 ? lo_halo : hi_halo)) FAIL(LBM_ERR_ARG, "no neighbour on side %d", side);
+        if (!has_nb(side)) FAIL(LBM_ERR_ARG, "no neighbour on side %d", side);
         CK(cudaSetDevice(d.device));
         mail_G = box.px + 32, mail_ms = box.plane + 2 * mail_G;
-        if (!d_mail[side]) {
-            if (dalloc(&d_mail[side], (size_t)mail_ms * 10)) return LBM_ERR_NOMEM;
-            CK(cudaMemsetAsync(d_mail[side], 0, (size_t)mail_ms * 10 * sizeof(T), st));
+        T *&mail = face[side].mail;
+        if (!mail) {
+            if (dalloc(&mail, (size_t)mail_ms * 10)) return LBM_ERR_NOMEM;
+            CK(cudaMemsetAsync(mail, 0, (size_t)mail_ms * 10 * sizeof(T), st));
         }
         if (h) {
             cudaIpcMemHandle_t ih;
-            CK(cudaIpcGetMemHandle(&ih, d_mail[side]));
+            CK(cudaIpcGetMemHandle(&ih, mail));
             memset(h, 0, sizeof(lbm_ipc_handle));
             memcpy(h, &ih, sizeof ih);
         }
-        if (ptr) *ptr = d_mail[side];
+        if (ptr) *ptr = mail;
         if (boff) {
-            int r = alloc_offset(d_mail[side], boff);
+            int r = alloc_offset(mail, boff);
             if (r) return r;
         }
         if (ms) *ms = mail_ms;
         if (guard) *guard = mail_G;
         return 0;
     }
-    // peer_mail: the NEIGHBOUR's mailbox of the side facing this slab, as mapped here (null detaches).  From now on
-    // this slab reads the entering populations of that face from its own mailbox and stores the leaving ones into
-    // the neighbour's: both sides of a face must switch together, between two steps.
+    // peer_mail: the NEIGHBOUR's mailbox of the side facing this slab, as mapped here (null detaches a mailbox link of
+    // either kind).  From now on this slab reads the entering populations of that face from its own mailbox and
+    // stores the leaving ones into the neighbour's: both sides of a face must switch together, between two steps.
     int mail_attach(int side, void *pm) override {
         if (side < 0 || side > 1) FAIL(LBM_ERR_ARG, "side must be 0 or 1");
-        if (!have_init || (pm && !d_mail[side])) FAIL(LBM_ERR_STATE, "lbm_mail_attach before lbm_mail_export of that side");
-        CK(cudaSetDevice(d.device));
-        CK(cudaStreamSynchronize(st));
-        if (pm && !mail_live[side]) {
-            int r = mail_move(side, 0);
-            if (r) return r;
-            mail_live[side] = true;
-        } else if (!pm && mail_live[side]) {
-            int r = mail_move(side, 1);
-            if (r) return r;
-            mail_live[side] = false;
-        }
-        peer_mail[side] = (T *)pm;
-        mail_staged[side] = false;
-        CK(cudaStreamSynchronize(st));
+        if (!have_init || (pm && !face[side].mail)) FAIL(LBM_ERR_STATE, "lbm_mail_attach before lbm_mail_export of that side");
+        if (!pm && !face[side].mailbox()) return 0;
+        int r = relink(side, pm ? Link::MAILBOX : Link::PACKED);
+        if (r) return r;
+        face[side].peer_mail = (T *)pm;
+        return 0;
+    }
+    // pa / pb: the neighbour's two population buffers as mapped here (both null detach a peer-buffer link)
+    int p2p_attach(int side, void *pa, void *pb, int64_t pqs, int64_t pc0, int64_t pown) override {
+        if (side < 0 || side > 1) FAIL(LBM_ERR_ARG, "side must be 0 or 1");
+        if (!have_init) FAIL(LBM_ERR_STATE, "p2p_attach before initialize");
+        if (!has_nb(side)) FAIL(LBM_ERR_ARG, "no neighbour on side %d", side);
+        if ((pa == nullptr) != (pb == nullptr)) FAIL(LBM_ERR_ARG, "both peer buffers or none");
+        Face &f = face[side];
+        if (!pa && f.kind != Link::PEER_BUFFERS) return 0;
+        int r = relink(side, pa ? Link::PEER_BUFFERS : Link::PACKED);
+        if (r) return r;
+        f.peer_buf[0] = (T *)pa, f.peer_buf[1] = (T *)pb, f.peer_qs = pqs, f.peer_c0 = pc0, f.peer_own = pown;
         return 0;
     }
     // Mailbox transport WITHOUT peer mapping: the leaving populations of this side go into a local staging buffer
@@ -1163,13 +1206,13 @@ struct Solver final : SolverBase {
     int mail_stage(int side) override {
         int r = mail_export(side, nullptr, nullptr, nullptr, nullptr, nullptr);
         if (r) return r;
+        Face &f = face[side];
         const size_t n = (size_t)mail_ms * 10;
-        if (!d_stage_out[side] && (dalloc(&d_stage_out[side], n) || dalloc(&d_stage_in[side], n))) return LBM_ERR_NOMEM;
-        CK(cudaMemsetAsync(d_stage_out[side], 0xFF, n * sizeof(T), st));
-        CK(cudaMemsetAsync(d_stage_in[side], 0xFF, n * sizeof(T), st));
-        r = mail_attach(side, d_stage_out[side]);
-        if (r) return r;
-        mail_staged[side] = true;
+        if (!f.stage_out && (dalloc(&f.stage_out, n) || dalloc(&f.stage_in, n))) return LBM_ERR_NOMEM;
+        CK(cudaMemsetAsync(f.stage_out, 0xFF, n * sizeof(T), st));
+        CK(cudaMemsetAsync(f.stage_in, 0xFF, n * sizeof(T), st));
+        if ((r = relink(side, Link::STAGED_MAILBOX))) return r;
+        f.peer_mail = f.stage_out;
         return 0;
     }
     int sync_export(lbm_ipc_handle *h, void **ptr, int64_t *boff) override {
@@ -1191,11 +1234,11 @@ struct Solver final : SolverBase {
     // effect: both sides reset their counters here, so attach on all slabs before any of them steps.
     int sync_attach(int side, void *peer) override {
         if (side < 0 || side > 1) FAIL(LBM_ERR_ARG, "side must be 0 or 1");
-        if (!(side == 0 ? lo_halo : hi_halo)) FAIL(LBM_ERR_ARG, "no neighbour on side %d", side);
+        if (!has_nb(side)) FAIL(LBM_ERR_ARG, "no neighbour on side %d", side);
         CK(cudaSetDevice(d.device));
         CK(cudaStreamSynchronize(st));
         // this slab is the HIGH neighbour of the slab below it and the LOW neighbour of the one above
-        peer_sync[side] = peer ? (unsigned long long *)peer + (side == 0 ? 1 : 0) : nullptr;
+        face[side].peer_sync = peer ? (unsigned long long *)peer + (side == 0 ? 1 : 0) : nullptr;
         CK(cudaMemsetAsync(d_sync + side, 0, sizeof(unsigned long long), st));
         CK(cudaMemsetAsync(d_sync + 2, 0, sizeof(unsigned long long), st));
         CK(cudaStreamSynchronize(st));
@@ -1260,7 +1303,7 @@ struct Solver final : SolverBase {
         if (!path) FAIL(LBM_ERR_ARG, "null path");
         CK(cudaSetDevice(d.device));
         {
-            int r = mail_drain();  // the population buffer is complete again; mail_refill() below hands the slots back
+            int r = mail_place_all(false);  // the population buffer is whole again; done() hands the slots back
             if (r) return r;
         }
         CK(cudaStreamSynchronize(st));
@@ -1282,7 +1325,7 @@ struct Solver final : SolverBase {
         int rc = 0;
         auto done = [&](int code, const std::string &msg) {
             if (have_init) {  // hand the mailbox slots back whatever happened to the file
-                const int r2 = mail_refill();
+                const int r2 = mail_place_all(true);
                 if (!code) code = r2;
             }
             if (f) fclose(f);
@@ -1376,29 +1419,21 @@ struct Solver final : SolverBase {
         }
         return 0;
     }
-    int p2p_attach(int side, void *pa, void *pb, int64_t pqs, int64_t pc0, int64_t pown) override {
-        if (side < 0 || side > 1) FAIL(LBM_ERR_ARG, "side must be 0 or 1");
-        if (!have_init) FAIL(LBM_ERR_STATE, "p2p_attach before initialize");
-        if (!(side == 0 ? lo_halo : hi_halo)) FAIL(LBM_ERR_ARG, "no neighbour on side %d", side);
-        if ((pa == nullptr) != (pb == nullptr)) FAIL(LBM_ERR_ARG, "both peer buffers or none");
-        peer_buf[side][0] = (T *)pa, peer_buf[side][1] = (T *)pb;
-        peer_qs[side] = pqs, peer_c0[side] = pc0, peer_own[side] = pown;
-        return 0;
-    }
     int halo_buffers(int side, void **send, void **recv, size_t *send_bytes, size_t *recv_bytes) override {
         if (side < 0 || side > 1) FAIL(LBM_ERR_ARG, "side must be 0 or 1");
         if (!have_init) FAIL(LBM_ERR_STATE, "halo_buffers before initialize");
-        const bool present = side == 0 ? lo_halo : hi_halo;
-        if (present && mail_staged[side]) {  // the part of the current step's parity: A on even, B on odd steps
+        const bool present = has_nb(side);
+        const Face &f = face[side];
+        if (present && f.kind == Link::STAGED_MAILBOX) {  // the part of the current step's parity: A on even, B on odd steps
             const size_t off = (steps & 1) ? (size_t)mail_ms * 5 : 0, bytes = (size_t)mail_ms * 5 * sizeof(T);
-            if (send) *send = d_stage_out[side] + off;
-            if (recv) *recv = d_stage_in[side] + off;
+            if (send) *send = f.stage_out + off;
+            if (recv) *recv = f.stage_in + off;
             if (send_bytes) *send_bytes = bytes;
             if (recv_bytes) *recv_bytes = bytes;
             return 0;
         }
-        if (send) *send = present ? d_send[side] : nullptr;
-        if (recv) *recv = present ? d_recv[side] : nullptr;
+        if (send) *send = present ? f.send : nullptr;
+        if (recv) *recv = present ? f.recv : nullptr;
         const size_t dense_b = (size_t)box.plane * 5 * sizeof(T);
         if (send_bytes) *send_bytes = !present ? 0 : (sparse ? (size_t)face_n[side] * 5 * sizeof(T) : dense_b);
         if (recv_bytes) *recv_bytes = !present ? 0 : (sparse ? (size_t)halo_n[side] * 5 * sizeof(T) : dense_b);
@@ -1517,12 +1552,12 @@ struct Solver final : SolverBase {
         if (!have_init) FAIL(LBM_ERR_STATE, "get_populations before initialize");
         CK(cudaSetDevice(d.device));
         {
-            int r = mail_drain();
+            int r = mail_place_all(false);
             if (r) return r;
         }
         struct Refill {
             Solver *s;
-            ~Refill() { s->mail_refill(); }
+            ~Refill() { s->mail_place_all(true); }
         } refill{this};
         const size_t n = (size_t)stored_own;
         if (d.storage == LBM_STORE_SPARSE_AA) {

@@ -90,7 +90,6 @@ class SlabCase(api.Case):
         self._p2p = False
         self._sync_ptrs = []
         self.timing = {}         # seconds spent in the phases of setup / enable_p2p (bench.py reports them)
-        self.no_mailboxes = False  # True: the dense in-place storage maps the neighbours' whole buffers like the others
         self._mapped = []        # IPC handles this rank holds a mapping of
         self.p2p_error = None    # why enable_p2p fell back, if it did
 
@@ -122,102 +121,60 @@ class SlabCase(api.Case):
         self.timing.update(geo_pre=t1 - t0, count_exchange=t2 - t1, index_init=time.perf_counter() - t2)
 
     def enable_p2p(self):
-        """Fused halo exchange: every rank maps its neighbours' population buffers and sync blocks (CUDA
-        IPC over NVLink); the step kernel stores the crossing populations there itself and the slabs
-        order their steps through progress flags in that memory (lbm_slab_step) -- no collective is
-        left in the time loop."""
-        import torch
-        import torch.distributed as dist
+        """Fused halo exchange: every rank maps what its neighbours export for it and their sync blocks (CUDA IPC
+        over NVLink); the step kernel stores the crossing populations there itself and the slabs order their steps
+        through progress flags in that memory (lbm_slab_step) -- no collective is left in the time loop.
 
-        import time
-
-        if self.desc.storage == api.STORE_DENSE_AA and not self.no_mailboxes:
-            return self._enable_mailboxes()
-        t0 = time.perf_counter()
-        mine = self.p2p_export()
-        mine.pop("ptrs")  # raw pointers mean nothing in another process
-        sy = self.sync_export()
-        # fixed-size record, one all_gather of bytes (no pickling): 3 IPC handles + 8 int64
-        rec = np.zeros(3 * 64 + 8 * 8, dtype=np.uint8)
-        rec[0:64] = np.frombuffer(mine["handles"][0], dtype=np.uint8)
-        rec[64:128] = np.frombuffer(mine["handles"][1], dtype=np.uint8)
-        rec[128:192] = np.frombuffer(sy["handle"], dtype=np.uint8)
-        rec[192:].view(np.int64)[:] = [mine["boff"][0], mine["boff"][1], sy["boff"], mine["qs"], mine["halo_c0"][0],
-                                       mine["halo_c0"][1], mine["face_c0"][0], mine["face_c0"][1]]
-        t = torch.from_numpy(rec).cuda()
-        allt = torch.empty(self.world * rec.size, dtype=torch.uint8, device="cuda")
-        dist.all_gather_into_tensor(allt, t, group=self.group)
-        allr = allt.cpu().numpy().reshape(self.world, rec.size)
-        t1 = time.perf_counter()
-        ok, attached = 1, []
-        try:
-            for side, nb in ((0, self.rank - 1), (1, self.rank + 1)):
-                if 0 <= nb < self.world:
-                    r = allr[nb]
-                    hs = [r[0:64].tobytes(), r[64:128].tobytes(), r[128:192].tobytes()]
-                    boff_a, boff_b, boff_s, qs, h0, h1, f0, f1 = (int(v) for v in r[192:].view(np.int64))
-                    ptrs = []
-                    for h, o in zip(hs, (boff_a, boff_b, boff_s)):
-                        ptrs.append(api.p2p_open(h) + o)
-                        self._mapped.append(h)
-                    # my low face feeds the neighbour's HIGH halo plane and vice versa
-                    self.p2p_attach(side, ptrs[0], ptrs[1], qs, (h0, h1)[1 - side], (f0, f1)[1 - side])
-                    attached.append((side, ptrs[2]))
-        except api.LbmError as e:
-            ok, self.p2p_error = 0, str(e)
-        # all ranks or none: a rank that cannot map its neighbour (no peer access / IPC) sends everyone
-        # back to the pack + NCCL path
-        flag = torch.tensor([ok], device="cuda")
-        dist.all_reduce(flag, op=dist.ReduceOp.MIN, group=self.group)
-        if int(flag.item()) == 0:
-            for side, _ in attached:
-                self.p2p_attach(side, None, None)
-            self._release_mappings()
-            return False
-        t2 = time.perf_counter()
-        self._sync_ptrs = attached
-        self._attach_sync()
-        self._p2p = True
-        self.timing.update(handle_exchange=t1 - t0, ipc_open=t2 - t1, sync_attach=time.perf_counter() - t2)
-        return True
-
-    def _enable_mailboxes(self):
-        """Dense in-place storage: neighbours exchange through small per-face mailboxes (lbm_mail_export / attach)
-        instead of mapping each other's whole population buffer -- cudaIpcOpenMemHandle costs 50-65 ms per GB mapped,
-        0.74 s for a 512^3 fp64 slab, against a few ms for the ~80 MB mailbox of a 1024^2 face."""
+        The dense in-place storage exports small per-face mailboxes (lbm_mail_export / attach), the other storages
+        their whole population buffers (lbm_p2p_export / attach): cudaIpcOpenMemHandle costs 50-65 ms per GB mapped,
+        0.74 s for a 512^3 fp64 slab, against a few ms for the ~80 MB mailbox of a 1024^2 face.  Returns False on
+        every rank, with nothing attached, when any rank cannot map its neighbours."""
         import time
 
         import torch
         import torch.distributed as dist
 
         t0 = time.perf_counter()
+        mail = self.desc.storage == api.STORE_DENSE_AA
         sides = [s for s, nb in ((0, self.rank - 1), (1, self.rank + 1)) if 0 <= nb < self.world]
-        rec = np.zeros(3 * 64 + 3 * 8, dtype=np.uint8)  # mailbox low, mailbox high, sync block: handle + byte offset each
-        offs = rec[192:].view(np.int64)
-        for s in sides:
-            m = self.mail_export(s)
-            rec[64 * s:64 * s + 64] = np.frombuffer(m["handle"], dtype=np.uint8)
-            offs[s] = m["boff"]
+        # fixed-size record, one all_gather of bytes (no pickling): 3 IPC handles (mailbox low / high or population
+        # buffer a / b, sync block), then 8 int64: their byte offsets, q stride, halo_c0[2], face_c0[2]
+        rec = np.zeros(3 * 64 + 8 * 8, dtype=np.uint8)
+        ints = rec[192:].view(np.int64)
+        if mail:
+            for s in sides:
+                m = self.mail_export(s)
+                rec[64 * s:64 * s + 64] = np.frombuffer(m["handle"], dtype=np.uint8)
+                ints[s] = m["boff"]
+        else:
+            e = self.p2p_export()
+            for k in (0, 1):
+                rec[64 * k:64 * k + 64] = np.frombuffer(e["handles"][k], dtype=np.uint8)
+            ints[:2], ints[3:] = e["boff"], [e["qs"], *e["halo_c0"], *e["face_c0"]]
         sy = self.sync_export()
         rec[128:192] = np.frombuffer(sy["handle"], dtype=np.uint8)
-        offs[2] = sy["boff"]
+        ints[2] = sy["boff"]
         t = torch.from_numpy(rec).cuda()
         allt = torch.empty(self.world * rec.size, dtype=torch.uint8, device="cuda")
         dist.all_gather_into_tensor(allt, t, group=self.group)
         allr = allt.cpu().numpy().reshape(self.world, rec.size)
         t1 = time.perf_counter()
-        ok, mails, syncs = 1, [], []
+        ok, links = 1, []
         try:
             for s in sides:
                 r = allr[self.rank - 1 if s == 0 else self.rank + 1]
-                o = r[192:].view(np.int64)
-                hm, hs = r[64 * (1 - s):64 * (1 - s) + 64].tobytes(), r[128:192].tobytes()  # the neighbour's FACING side
-                mails.append((s, api.p2p_open(hm) + int(o[1 - s])))
-                self._mapped.append(hm)
-                syncs.append((s, api.p2p_open(hs) + int(o[2])))
-                self._mapped.append(hs)
+                o = [int(v) for v in r[192:].view(np.int64)]
+                # the neighbour's mailbox of the side FACING this slab, or both its buffers; then its sync block
+                ptrs = []
+                for k in ((1 - s,) if mail else (0, 1)) + (2,):
+                    h = r[64 * k:64 * k + 64].tobytes()
+                    ptrs.append(api.p2p_open(h) + o[k])
+                    self._mapped.append(h)
+                links.append((s, ptrs, o))
         except api.LbmError as e:
             ok, self.p2p_error = 0, str(e)
+        # all ranks or none: a rank that cannot map its neighbour (no peer access / IPC) sends everyone
+        # back to the pack / staged path
         flag = torch.tensor([ok], device="cuda")
         dist.all_reduce(flag, op=dist.ReduceOp.MIN, group=self.group)
         if int(flag.item()) == 0:
@@ -225,9 +182,12 @@ class SlabCase(api.Case):
             return False
         t2 = time.perf_counter()
         dist.barrier(group=self.group)  # both slabs of a face switch over between the same two steps
-        for s, ptr in mails:
-            self.mail_attach(s, ptr)
-        self._sync_ptrs = syncs
+        for s, ptrs, o in links:
+            if mail:
+                self.mail_attach(s, ptrs[0])
+            else:  # my low face feeds the neighbour's HIGH halo plane and vice versa
+                self.p2p_attach(s, ptrs[0], ptrs[1], o[3], o[5 - s], o[7 - s])
+        self._sync_ptrs = [(s, ptrs[-1]) for s, ptrs, _ in links]
         self._attach_sync()
         self._p2p = True
         self.timing.update(handle_exchange=t1 - t0, ipc_open=t2 - t1, sync_attach=time.perf_counter() - t2)

@@ -201,6 +201,25 @@ def rel_err(got, ref):
     return max(e_u / scale, e_r)
 
 
+def virtual_slabs(name, n, P):
+    """P dense in-place slab handles of one case on ONE GPU, initialised, numbered like the single domain"""
+    import lattice_boltzmann_method_gpu_b200 as L
+    from lattice_boltzmann_method_gpu_b200 import slab
+
+    nz = {"ldc": n, "pos": n, "bif": 32, "cor": 44, "corstep": 28}[name]
+    cs = [gpu_case(name, n, L.F64, L.MATH_FAST, z_range=r, storage=L.STORE_DENSE_AA) for r in slab.slab_ranges(nz, P)]
+    for c in cs:
+        c.geo_pre()
+    offs, total = slab.compact_offsets([c.local_stored_count() for c in cs])
+    for c, o in zip(cs, offs):
+        c.set_compact_offset(o, total)
+        c.index_transform()
+        if name == "bif":
+            c.set_bc_planes(*bif_bc_planes())
+        c.initialize()
+    return cs
+
+
 def attach_virtual_slabs(cs, mail=False):
     """several slab handles on ONE GPU: every handle stores its crossing populations straight into its
     neighbours' buffers (lbm_p2p_attach with plain device pointers) or, mail=True, into their mailboxes

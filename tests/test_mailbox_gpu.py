@@ -11,24 +11,6 @@ import helpers as H
 pytestmark = pytest.mark.gpu
 
 
-def _slabs(name, n, P, L, prec=None):
-    from lattice_boltzmann_method_gpu_b200 import slab
-
-    nz = {"ldc": n, "pos": n, "bif": 32, "cor": 44, "corstep": 28}[name]
-    cs = [H.gpu_case(name, n, L.F64 if prec is None else prec, L.MATH_FAST, z_range=r, storage=L.STORE_DENSE_AA)
-          for r in slab.slab_ranges(nz, P)]
-    for c in cs:
-        c.geo_pre()
-    offs, total = slab.compact_offsets([c.local_stored_count() for c in cs])
-    for c, o in zip(cs, offs):
-        c.set_compact_offset(o, total)
-        c.index_transform()
-        if name == "bif":
-            c.set_bc_planes(*H.bif_bc_planes())
-        c.initialize()
-    return cs
-
-
 @pytest.mark.parametrize("name,n,P", [("ldc", 24, 3), ("bif", None, 4), ("cor", None, 5), ("pos", 24, 2), ("ldc", 12, 12),
                                       ("ldc", 12, 6), ("corstep", None, 7)])
 def test_mailbox_slabs_equal_single_domain_bitwise(name, n, P):
@@ -36,7 +18,7 @@ def test_mailbox_slabs_equal_single_domain_bitwise(name, n, P):
 
     one = H.gpu_case(name, n, L.F64, L.MATH_FAST, storage=L.STORE_DENSE_AA)
     H.gpu_setup(one, name)
-    cs = _slabs(name, n, P, L)
+    cs = H.virtual_slabs(name, n, P)
     H.attach_virtual_slabs(cs, mail=True)
     for steps in (1, 1, 1, 18):  # totals 1, 2, 3, 21
         one.step(steps)
@@ -54,7 +36,7 @@ def test_mailbox_checkpoint_populations_and_switching_back(tmp_path):
     H.gpu_setup(one, name)
     one.step(30)
     ref = one.get_fields()
-    cs = _slabs(name, n, P, L)
+    cs = H.virtual_slabs(name, n, P)
     H.attach_virtual_slabs(cs, mail=True)
     H.step_virtual_slabs(cs, 7)
     pops = [c.get_populations() for c in cs]      # drains and refills the mailboxes around the gather
@@ -78,7 +60,7 @@ def test_mailbox_checkpoint_populations_and_switching_back(tmp_path):
     for k in range(4):
         assert np.array_equal(np.concatenate([c.get_fields()[k] for c in cs]), ref[k]), k
     # a checkpoint written with mailboxes loads into a fresh set of slabs without
-    ds = _slabs(name, n, P, L)
+    ds = H.virtual_slabs(name, n, P)
     H.attach_virtual_slabs(ds, mail=False)
     for r, c in enumerate(ds):
         c.checkpoint_load(tmp_path / f"ck{r}.bin")
