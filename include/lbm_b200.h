@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define LBM_B200_ABI_VERSION 2
+#define LBM_B200_ABI_VERSION 3
 
 typedef struct lbm_solver_s *lbm_handle;
 
@@ -73,6 +73,12 @@ typedef enum {
     LBM_MATH_FAST = 0,   /* FMA-contracted, reciprocal-multiply BGK (default, the measured path) */
     LBM_MATH_STRICT = 1  /* the reference's expression order, no contraction: bit-identical to the CPU oracle */
 } lbm_math;
+
+/* collision operator of the fused kernel (lbm_set_collision) */
+typedef enum {
+    LBM_COLL_BGK = 0, /* single relaxation time 1/tau (default, the reference's operator) */
+    LBM_COLL_TRT = 1  /* two relaxation times: even part 1/tau, odd part set by the magic parameter; FAST only */
+} lbm_collision;
 
 /* boundary-condition kinds of the non-equilibrium extrapolation (SURVEY A.4) */
 typedef enum {
@@ -353,6 +359,8 @@ int lbm_group_output_save(lbm_group g, int32_t t); /* ASCII: ONE file, byte-iden
 int lbm_group_run_fixed(lbm_group g, int32_t repeat, int32_t time_save, int32_t write_files);
 int lbm_group_run_converge(lbm_group g, int32_t max_it, double tol, int32_t stag_max, int32_t time_save,
                            int32_t write_files, int32_t *iterations, double *residual);
+/* lbm_set_collision on every slab of the group (all or none: the arguments are checked before any slab changes) */
+int lbm_group_set_collision(lbm_group g, int32_t model, double magic);
 
 /* Tuning knobs that are not part of a case description.  "persistent": 1 runs batches of steps of the in-place
  * sparse storage in one cooperative launch with a grid barrier between steps (for grids that live in L2); 0 or
@@ -361,6 +369,28 @@ int lbm_group_run_converge(lbm_group g, int32_t max_it, double tol, int32_t stag
  * serialization, so that a step's launch latency and geometry loads overlap the previous step's tail (a 64^3
  * step: 9.9 -> 7.6 us); 0 serialises launches the ordinary way.  Single-domain handles only. */
 int lbm_set_option(lbm_handle h, const char *name, double value);
+
+/* Collision operator.  LBM_COLL_BGK (the default; a handle that never calls this steps exactly as before):
+ *     f_q <- f_q - (f_q - feq_q) / tau.
+ * LBM_COLL_TRT, two relaxation times (Ginzburg, Verhaeghe & d'Humieres, Commun. Comput. Phys. 3, 2008): with
+ * the opposite direction qbar of q,
+ *     n+ = (f_q + f_qbar)/2 - (feq_q + feq_qbar)/2      n- = (f_q - f_qbar)/2 - (feq_q - feq_qbar)/2
+ *     f_q <- f_q - om+ n+ - om- n-                      f_0 <- f_0 - om+ (f_0 - feq_0)
+ * om+ = 1/tau sets the viscosity as for BGK; om- = 1 / (1/2 + magic / (tau - 1/2)), i.e. the magic parameter
+ * Lambda = (1/om+ - 1/2)(1/om- - 1/2) = magic.  At fixed Lambda the steady bounce-back solution does not depend on
+ * tau: Lambda = 3/16 puts a straight wall exactly half-way for Poiseuille flow, Lambda = 1/4 is the usual choice
+ * for stability.  Lambda = (tau - 1/2)^2 gives om- = om+, i.e. BGK.
+ * Inlet / outlet / lid links under TRT: the node's post-collision non-equilibrium n_q = g_q - feq_q(rho_x, u_x) is
+ * split with the opposite link and relaxed like the collision,
+ *     feq_q(rho_bc, u_bc) + (1 - om+) (n_q + n_qbar)/2 + (1 - om-) (n_q - n_qbar)/2,
+ * which is the BGK rule feq_q(rho_bc, u_bc) + n_q (1 - 1/tau) when om- = om+.  Bounce-back and static links are
+ * unchanged.  TRT exists in LBM_MATH_FAST arithmetic only (STRICT is the reference's expression order, and the
+ * reference has no TRT).
+ * Callable any time after lbm_create; takes effect from the next step.  LBM_ERR_STATE inside lbm_step_begin ..
+ * lbm_step_end; LBM_ERR_ARG for an unknown model, a magic parameter that is not finite and > 0 (TRT; ignored for
+ * BGK), tau <= 1/2 with TRT, or TRT on an LBM_MATH_STRICT handle -- the handle then keeps its operator.
+ * Checkpoints of a TRT run carry the operator and Lambda: only a handle with the same ones loads them. */
+int lbm_set_collision(lbm_handle h, int32_t model, double magic);
 
 /* Self-checking build of the library (-DLBM_SELFCHECK; tools/selfcheck.py builds and runs it -- the stand-in for
  * compute-sanitizer, which the GPU pool does not offer): out[0] = population accesses of the step kernels that

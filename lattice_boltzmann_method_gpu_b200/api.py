@@ -28,6 +28,7 @@ CASE_LDC, CASE_POISEUILLE, CASE_GEO_Y_INOUT, CASE_GEO_OPENINGS = 0, 1, 2, 3
 F32, F64 = 0, 1
 STORE_DENSE_AB, STORE_DENSE_AA, STORE_SPARSE_AB, STORE_SPARSE_AA = 0, 1, 2, 3
 MATH_FAST, MATH_STRICT = 0, 1
+COLL_BGK, COLL_TRT = 0, 1
 BC_NONE, BC_V, BC_P, BC_VP = 0, 1, 2, 3
 SRC_CONST, SRC_PARABOLA, SRC_PLANE_INLET, SRC_PLANE_OUTLET = 0, 1, 2, 3
 RES_VELSUM, RES_U2SUM = 0, 1
@@ -80,10 +81,11 @@ ABI_SYMBOLS = [
     "lbm_step_begin", "lbm_step_interior", "lbm_step_end", "lbm_last_velsum", "lbm_stream", "lbm_sync",
     "lbm_p2p_export", "lbm_p2p_open", "lbm_p2p_close", "lbm_p2p_attach", "lbm_checkpoint_save", "lbm_checkpoint_load",
     "lbm_slab_step", "lbm_sync_export", "lbm_sync_attach", "lbm_mail_export", "lbm_mail_attach", "lbm_mail_stage", "lbm_write_bc_csv", "lbm_debug_selfcheck", "lbm_set_option",
+    "lbm_set_collision",
     "lbm_create_distributed", "lbm_group_destroy", "lbm_group_last_error", "lbm_group_size", "lbm_group_slab",
     "lbm_group_setup", "lbm_group_step", "lbm_group_num_fluid", "lbm_group_residual", "lbm_group_get_fields",
     "lbm_group_get_index", "lbm_group_set_output_format", "lbm_group_output_save", "lbm_group_run_fixed",
-    "lbm_group_run_converge",
+    "lbm_group_run_converge", "lbm_group_set_collision",
 ]
 
 _lib = None
@@ -161,6 +163,7 @@ def load_library() -> C.CDLL:
         "lbm_write_bc_csv": ([vp, C.c_char_p], C.c_int),
         "lbm_debug_selfcheck": ([vp, vp], C.c_int),
         "lbm_set_option": ([vp, C.c_char_p, dbl], C.c_int),
+        "lbm_set_collision": ([vp, i32, dbl], C.c_int),
         "lbm_create_distributed": ([P(CaseDesc), i32, vp, P(vp)], C.c_int),
         "lbm_group_destroy": ([vp], C.c_int),
         "lbm_group_last_error": ([vp], C.c_char_p),
@@ -176,6 +179,7 @@ def load_library() -> C.CDLL:
         "lbm_group_output_save": ([vp, i32], C.c_int),
         "lbm_group_run_fixed": ([vp, i32, i32, i32], C.c_int),
         "lbm_group_run_converge": ([vp, i32, dbl, i32, i32, i32, P(i32), P(dbl)], C.c_int),
+        "lbm_group_set_collision": ([vp, i32, dbl], C.c_int),
     }
     for name, (args, res) in sig.items():
         fn = getattr(L, name)
@@ -368,6 +372,11 @@ class Case:
     def set_option(self, name: str, value: float):
         self._ck(self._L.lbm_set_option(self._h, name.encode(), float(value)))
 
+    def set_collision(self, model: int, magic: float = 3 / 16):
+        """COLL_BGK (default) or COLL_TRT with the magic parameter Lambda (3/16: a straight bounce-back wall lies
+        exactly half-way; 1/4: the usual choice for stability).  FAST arithmetic only; from the next step on."""
+        self._ck(self._L.lbm_set_collision(self._h, int(model), float(magic)))
+
     def selfcheck(self):
         """(out-of-range accesses, elements touched by two threads in one launch, launches checked) of a
         self-checking build; raises LbmError on a normal build"""
@@ -532,6 +541,10 @@ class Group:
 
     def set_output_format(self, fmt: int):
         self._ck(self._L.lbm_group_set_output_format(self._g, fmt))
+
+    def set_collision(self, model: int, magic: float = 3 / 16):
+        """Case.set_collision on every slab"""
+        self._ck(self._L.lbm_group_set_collision(self._g, int(model), float(magic)))
 
     def outputSave(self, t: int):
         self._ck(self._L.lbm_group_output_save(self._g, int(t)))

@@ -1,4 +1,4 @@
-// D3Q19 lattice constants and the per-node BGK arithmetic, device side.
+// D3Q19 lattice constants and the per-node collision arithmetic (BGK, TRT), device side.
 //
 // Lattice numbering, weights and opposite pairs follow the reference's pull
 // offsets and swap list (ldc.cu:184-201, 207-313, 320-322; SURVEY A.1).
@@ -158,6 +158,29 @@ __device__ __forceinline__ double rho_over<double>(double r, int d) {
 }
 
 // ---------------------------------------------------------------------------
+// moments of one node in FAST arithmetic, shared by both FAST collisions (collide_bgk, collide_trt).
+// ---------------------------------------------------------------------------
+template <typename T>
+__device__ __forceinline__ void moments_fast(const T (&f)[Q], T &rho, T &ux, T &uy, T &uz) {
+    // pairwise sums shorten the dependency chains; order is free in FAST mode.
+    // Every multiply-add below is an EXPLICIT fma and the translation unit is compiled with -fmad=false
+    // like the STRICT one: which operations fuse is then decided here, not by ptxas per kernel
+    // instantiation, so all storages, the persistent kernel, the two-segment kernel and the slab (peer
+    // store) variants produce the same bits from the same inputs -- "N slabs == 1 domain" and
+    // "in-place == two buffers" hold bit for bit in FAST arithmetic too.
+    T a0 = f[1] + f[2], a1 = f[3] + f[4], a2 = f[5] + f[6];
+    T d0 = f[7] + f[10], d1 = f[8] + f[9], d2 = f[11] + f[14], d3 = f[12] + f[13], d4 = f[15] + f[18],
+      d5 = f[16] + f[17];
+    T r = ((f[0] + a0) + (a1 + a2)) + ((d0 + d1) + (d2 + d3)) + (d4 + d5);
+    T inv = T(1.0) / r;
+    T mx = ((f[1] - f[2]) + (f[7] - f[10])) + ((f[8] - f[9]) + (f[11] - f[14])) + (f[12] - f[13]);
+    T my = ((f[3] - f[4]) + (f[7] - f[10])) + ((f[9] - f[8]) + (f[15] - f[18])) + (f[17] - f[16]);
+    T mz = ((f[5] - f[6]) + (f[11] - f[14])) + ((f[13] - f[12]) + (f[15] - f[18])) + (f[16] - f[17]);
+    rho = r;
+    ux = mx * inv, uy = my * inv, uz = mz * inv;
+}
+
+// ---------------------------------------------------------------------------
 // moments + BGK collision of one node.  f[] in: post-streaming populations,
 // out: post-collision.  Moments returned are the pre-collision ones the
 // reference stores (bif.cu:574-595).
@@ -179,22 +202,8 @@ __device__ __forceinline__ void collide_bgk(T (&f)[Q], T tau, T inv_tau, T &rho,
             f[q] = f[q] - (f[q] - feq) / tau;
         }
     } else {
-        // pairwise sums shorten the dependency chains; order is free in FAST mode.
-        // Every multiply-add below is an EXPLICIT fma and the translation unit is compiled with -fmad=false
-        // like the STRICT one: which operations fuse is then decided here, not by ptxas per kernel
-        // instantiation, so all storages, the persistent kernel, the two-segment kernel and the slab (peer
-        // store) variants produce the same bits from the same inputs -- "N slabs == 1 domain" and
-        // "in-place == two buffers" hold bit for bit in FAST arithmetic too.
-        T a0 = f[1] + f[2], a1 = f[3] + f[4], a2 = f[5] + f[6];
-        T d0 = f[7] + f[10], d1 = f[8] + f[9], d2 = f[11] + f[14], d3 = f[12] + f[13], d4 = f[15] + f[18],
-          d5 = f[16] + f[17];
-        T r = ((f[0] + a0) + (a1 + a2)) + ((d0 + d1) + (d2 + d3)) + (d4 + d5);
-        T inv = T(1.0) / r;
-        T mx = ((f[1] - f[2]) + (f[7] - f[10])) + ((f[8] - f[9]) + (f[11] - f[14])) + (f[12] - f[13]);
-        T my = ((f[3] - f[4]) + (f[7] - f[10])) + ((f[9] - f[8]) + (f[15] - f[18])) + (f[17] - f[16]);
-        T mz = ((f[5] - f[6]) + (f[11] - f[14])) + ((f[13] - f[12]) + (f[15] - f[18])) + (f[16] - f[17]);
-        rho = r;
-        ux = mx * inv, uy = my * inv, uz = mz * inv;
+        moments_fast<T>(f, rho, ux, uy, uz);
+        const T r = rho;
         // f* = f + om (feq - f): the difference is formed first, like the reference's
         // f - (f - feq)/tau, so the rounding error scales with the (small) non-equilibrium
         // part.  The algebraically equal (1-om) f + om feq cancels two O(f) terms when
@@ -228,6 +237,54 @@ __device__ __forceinline__ void collide_bgk(T (&f)[Q], T tau, T inv_tau, T &rho,
         LBM_PAIR(17, 16, uy - uz, k2)
 #undef LBM_PAIR
     }
+}
+
+// ---------------------------------------------------------------------------
+// moments + two-relaxation-time (TRT) collision of one node, FAST arithmetic only (Ginzburg, Verhaeghe &
+// d'Humieres, Commun. Comput. Phys. 3, 2008).  For an opposite pair (q, qbar) the non-equilibrium splits
+// into an even and an odd part,
+//     n+ = (f_q + f_qbar)/2 - kw even      n- = (f_q - f_qbar)/2 - kw odd
+//     f_q <- f_q - om_p n+ - om_m n-       f_qbar <- f_qbar - om_p n+ + om_m n-
+// with the equilibrium parts even / odd of collide_bgk's LBM_PAIR.  om_p = 1/tau keeps the viscosity;
+// om_m is set by the host from the magic parameter Lambda = (1/om_p - 1/2)(1/om_m - 1/2).  Moments returned
+// are the pre-collision ones, as for collide_bgk.
+// ---------------------------------------------------------------------------
+template <typename T>
+__device__ __forceinline__ void collide_trt(T (&f)[Q], T om_p, T om_m, T &rho, T &ux, T &uy, T &uz) {
+    moments_fast<T>(f, rho, ux, uy, uz);
+    const T r = rho;
+    const T base = fma(T(-1.5), fma(ux, ux, fma(uy, uy, uz * uz)), T(1.0));
+    const T k0 = rho_over<T>(r, 3), k1 = rho_over<T>(r, 18), k2 = T(0.5) * k1;
+    f[0] = fma(om_p, fma(k0, base, -f[0]), f[0]);
+#define LBM_PAIR_TRT(qp, qm, cu, kw)                                  \
+    {                                                                 \
+        T cu_ = (cu);                                                 \
+        T even = fma(T(4.5) * cu_, cu_, base);                        \
+        T odd = T(3.0) * cu_;                                         \
+        T np = fma(-(kw), even, T(0.5) * (f[qp] + f[qm]));            \
+        T nm = fma(-(kw), odd, T(0.5) * (f[qp] - f[qm]));             \
+        T rp = om_p * np;                                             \
+        f[qp] = fma(-om_m, nm, f[qp] - rp);                           \
+        f[qm] = fma(om_m, nm, f[qm] - rp);                            \
+    }
+    LBM_PAIR_TRT(1, 2, ux, k1)
+    LBM_PAIR_TRT(3, 4, uy, k1)
+    LBM_PAIR_TRT(5, 6, uz, k1)
+    LBM_PAIR_TRT(7, 10, ux + uy, k2)
+    LBM_PAIR_TRT(8, 9, ux - uy, k2)
+    LBM_PAIR_TRT(11, 14, ux + uz, k2)
+    LBM_PAIR_TRT(12, 13, ux - uz, k2)
+    LBM_PAIR_TRT(15, 18, uy + uz, k2)
+    LBM_PAIR_TRT(17, 16, uy - uz, k2)
+#undef LBM_PAIR_TRT
+}
+
+// one collision of the fused step kernels, chosen at compile time: COLL is an lbm_collision value
+template <typename T, bool STRICT, int COLL>
+__device__ __forceinline__ void collide(T (&f)[Q], const StepParams<T> &p, T &rho, T &ux, T &uy, T &uz) {
+    static_assert(COLL == LBM_COLL_BGK || !STRICT, "TRT exists in FAST arithmetic only");
+    if constexpr (COLL == LBM_COLL_TRT) collide_trt<T>(f, p.inv_tau, p.om_m, rho, ux, uy, uz);
+    else collide_bgk<T, STRICT>(f, p.tau, p.inv_tau, rho, ux, uy, uz);
 }
 
 }  // namespace lbm

@@ -39,6 +39,17 @@ static std::string fmt(const char *f, ...) {
     return buf;
 }
 
+// the argument rules of lbm_set_collision (include/lbm_b200.h); empty: accepted
+static std::string collision_refusal(const lbm_case_desc &d, int model, double magic) {
+    if (model == LBM_COLL_BGK) return "";
+    if (model != LBM_COLL_TRT) return fmt("unknown collision model %d (LBM_COLL_BGK = 0, LBM_COLL_TRT = 1)", model);
+    if (!std::isfinite(magic) || !(magic > 0.0)) return fmt("TRT magic parameter must be finite and > 0 (got %g)", magic);
+    if (!(d.tau > 0.5)) return fmt("TRT needs tau > 1/2 (tau = %g)", d.tau);
+    if (d.math == LBM_MATH_STRICT)
+        return "TRT exists in LBM_MATH_FAST arithmetic only (STRICT is the reference's expression order, which has no TRT)";
+    return "";
+}
+
 struct SolverBase {
     virtual ~SolverBase() {}
     std::string err;
@@ -92,6 +103,7 @@ struct SolverBase {
     virtual void *stream_ptr() = 0;
     virtual int selfcheck(uint64_t *out2) = 0;
     virtual int set_option(const char *name, double value) = 0;
+    virtual int set_collision(int model, double magic) = 0;
     int64_t steps = 0, launches = 0, nfluid = 0, dev_bytes = 0;
 };
 
@@ -736,7 +748,7 @@ struct Solver final : SolverBase {
         const bool peers = lo_halo || hi_halo;
         CK(cudaSetDevice(d.device));
         if (d.math == LBM_MATH_STRICT) CK(preload_step_kernels_strict<T>(d.storage, speculative_pull(), peers, resid));
-        else CK(preload_step_kernels_fast<T>(d.storage, speculative_pull(), peers, resid));
+        else CK(preload_step_kernels_fast<T>(d.storage, speculative_pull(), peers, resid, collision));
         return 0;
     }
 
@@ -752,6 +764,11 @@ struct Solver final : SolverBase {
         p.tau = (T)d.tau;
         p.inv_tau = T(1.0) / p.tau;
         p.om1 = T(1.0) - T(1.0) / p.tau;
+        p.collision = collision;
+        if (collision == LBM_COLL_TRT) {
+            const double om_m = 1.0 / (0.5 + trt_magic / (d.tau - 0.5));  // Lambda = (1/om+ - 1/2)(1/om- - 1/2)
+            p.om_m = (T)om_m, p.om1_m = (T)(1.0 - om_m);
+        }
         double sc = 1.0;
         if (d.pulse_amp != 0.0) sc = 1.0 + d.pulse_amp * std::sin(2.0 * M_PI * (double)steps / d.pulse_period);
         p.pulse_scale = (T)sc;
@@ -816,6 +833,8 @@ struct Solver final : SolverBase {
     int sm_count = 0;
     static constexpr int PERSIST_MAX_STEPS = 2048, PERSIST_BAR_WORDS = 64 + 32 * 64;  // = BAR_WORDS of step_sparse_aa.cuh
     int opt_persist = -1;  // lbm_set_option("persistent", 0 / 1); -1: by size
+    int collision = LBM_COLL_BGK;  // lbm_set_collision
+    double trt_magic = 0.0;        // TRT: Lambda
     int opt_pdl = 1;       // lbm_set_option("overlap_launches", 0 / 1)
     bool use_persist() {
         if (d.storage != LBM_STORE_SPARSE_AA || lo_halo || hi_halo) return false;
@@ -1291,6 +1310,7 @@ struct Solver final : SolverBase {
         }
         mix(&nfluid, sizeof nfluid), mix(&stored_box, sizeof stored_box);
         if (have_planes) mix(h_in.data(), h_in.size() * sizeof(float)), mix(h_out.data(), h_out.size() * sizeof(float));
+        if (collision != LBM_COLL_BGK) mix(&collision, sizeof collision), mix(&trt_magic, sizeof trt_magic);  // BGK keeps its old hash
         *out = h;
         return 0;
     }
@@ -2057,6 +2077,13 @@ struct Solver final : SolverBase {
         chk_elems = elems;
         return 0;
     }
+    int set_collision(int model, double lambda) override {
+        if (in_step) FAIL(LBM_ERR_STATE, "lbm_set_collision inside lbm_step_begin / lbm_step_end");
+        const std::string why = collision_refusal(d, model, lambda);
+        if (!why.empty()) FAIL(LBM_ERR_ARG, "lbm_set_collision: %s", why.c_str());
+        collision = model, trt_magic = model == LBM_COLL_TRT ? lambda : 0.0;
+        return 0;
+    }
     int set_option(const char *name, double value) override {
         if (!strcmp(name, "persistent")) opt_persist = value < 0 ? -1 : (value != 0.0);
         else if (!strcmp(name, "overlap_launches")) opt_pdl = value != 0.0;
@@ -2318,6 +2345,7 @@ int lbm_mail_attach(lbm_handle h, int32_t side, void *peer_mail) { H_OR_FAIL; re
 int lbm_mail_stage(lbm_handle h, int32_t side) { H_OR_FAIL; return h->s->mail_stage(side); }
 int lbm_sync_attach(lbm_handle h, int32_t side, void *peer_sync) { H_OR_FAIL; return h->s->sync_attach(side, peer_sync); }
 int lbm_set_option(lbm_handle h, const char *name, double value) { H_OR_FAIL; return name ? h->s->set_option(name, value) : LBM_ERR_ARG; }
+int lbm_set_collision(lbm_handle h, int32_t model, double magic) { H_OR_FAIL; return h->s->set_collision(model, magic); }
 int lbm_debug_selfcheck(lbm_handle h, uint64_t out[3]) { H_OR_FAIL; return out ? h->s->selfcheck(out) : LBM_ERR_ARG; }
 int lbm_write_bc_csv(lbm_handle h, const char *path) { H_OR_FAIL; return path ? h->s->write_bc_csv(path) : LBM_ERR_ARG; }
 
@@ -2486,6 +2514,16 @@ int lbm_group_step(lbm_group g, int32_t n, float *elapsed_ms) {
         if ((rc = group_enqueue(g, i == n - 1 ? LBM_STEP_MOMENTS : 0, -1))) return rc;
     if ((rc = group_sync(g))) return rc;
     if (elapsed_ms) *elapsed_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    return LBM_OK;
+}
+int lbm_group_set_collision(lbm_group g, int32_t model, double magic) {
+    G_OR_FAIL;
+    const std::string why = lbm::collision_refusal(g->d, model, magic);  // every slab has the group's tau and math
+    if (!why.empty()) return g->fail(LBM_ERR_ARG, "lbm_group_set_collision: " + why);
+    for (size_t r = 0; r < g->h.size(); r++) {
+        const int rc = lbm_set_collision(g->h[r], model, magic);
+        if (rc) return g->from((int)r, rc);
+    }
     return LBM_OK;
 }
 int64_t lbm_group_num_fluid(lbm_group g) {

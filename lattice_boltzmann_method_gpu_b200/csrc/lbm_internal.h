@@ -104,6 +104,13 @@ struct StepParams {
     unsigned long long *chk_shadow[2];  // (launch id << 32) | (thread + 1) per buffer element
     unsigned long long *chk_count;      // [0] accesses outside the buffers, [1] elements touched by two threads in one launch
     unsigned int chk_launch;
+    // collision operator (lbm_collision) and, for TRT, its odd-part rate omega- and 1 - omega- (lattice.cuh
+    // collide_trt); the even-part rate is inv_tau.  Appended last so that no member above moves.
+    int collision;
+    T om_m, om1_m;
+    // SparseParams embeds this struct: its later members move by what was appended here.  A multiple of 16 bytes
+    // keeps their 16-byte alignment, which decides how the kernels merge parameter loads (LDCU.128).
+    int align16[sizeof(T) == 4 ? 2 : 4];
 };
 
 // Precomputed inlet / outlet links of the in-place sparse storage: per node with NODE_HAS_BC a header
@@ -256,7 +263,7 @@ cudaError_t launch_step_sparse_aa_fast(const SparseParams<T> &p, bool moments, b
 template <typename T>
 cudaError_t launch_step_sparse_aa_strict(const SparseParams<T> &p, bool moments, bool resid, cudaStream_t s);
 template <typename T>
-cudaError_t preload_step_kernels_fast(int storage, bool speculative, bool peers, bool resid);
+cudaError_t preload_step_kernels_fast(int storage, bool speculative, bool peers, bool resid, int collision);
 template <typename T>
 cudaError_t preload_step_kernels_strict(int storage, bool speculative, bool peers, bool resid);
 // nsteps steps of a single-domain in-place sparse handle in ONE cooperative launch (grids that live in L2)

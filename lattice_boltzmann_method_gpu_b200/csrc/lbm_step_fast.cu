@@ -44,13 +44,19 @@ template cudaError_t launch_sparse_aa_persist_fast<double>(const SparseParams<do
 
 namespace lbm {
 // loads the step kernels a run loop of this storage is about to launch (step_dense.cuh preload_kernel);
-// resid: the variants that sum |u| (lbm_run_converge) or those that do not (lbm_run_fixed)
-template <typename T>
-cudaError_t preload_step_kernels_fast(int storage, bool speculative, bool peers, bool resid) {
-    if (storage == LBM_STORE_SPARSE_AA) return preload_step_sparse_aa_impl<T, false>(peers, resid);
-    if (storage == LBM_STORE_SPARSE_AB) return preload_step_sparse_impl<T, false>(resid);
-    return preload_step_dense_impl<T, false>(storage, speculative, resid);
+// resid: the variants that sum |u| (lbm_run_converge) or those that do not (lbm_run_fixed); collision: those of
+// this lbm_collision
+template <typename T, int COLL>
+cudaError_t preload_step_kernels_coll(int storage, bool speculative, bool peers, bool resid) {
+    if (storage == LBM_STORE_SPARSE_AA) return preload_step_sparse_aa_impl<T, false, COLL>(peers, resid);
+    if (storage == LBM_STORE_SPARSE_AB) return preload_step_sparse_impl<T, false, COLL>(resid);
+    return preload_step_dense_impl<T, false, COLL>(storage, speculative, resid);
 }
-template cudaError_t preload_step_kernels_fast<float>(int, bool, bool, bool);
-template cudaError_t preload_step_kernels_fast<double>(int, bool, bool, bool);
+template <typename T>
+cudaError_t preload_step_kernels_fast(int storage, bool speculative, bool peers, bool resid, int collision) {
+    if (collision == LBM_COLL_TRT) return preload_step_kernels_coll<T, LBM_COLL_TRT>(storage, speculative, peers, resid);
+    return preload_step_kernels_coll<T, LBM_COLL_BGK>(storage, speculative, peers, resid);
+}
+template cudaError_t preload_step_kernels_fast<float>(int, bool, bool, bool, int);
+template cudaError_t preload_step_kernels_fast<double>(int, bool, bool, bool, int);
 }  // namespace lbm

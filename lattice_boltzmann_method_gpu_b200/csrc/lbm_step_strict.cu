@@ -50,9 +50,9 @@ namespace lbm {
 // resid: the variants that sum |u| (lbm_run_converge) or those that do not (lbm_run_fixed)
 template <typename T>
 cudaError_t preload_step_kernels_strict(int storage, bool speculative, bool peers, bool resid) {
-    if (storage == LBM_STORE_SPARSE_AA) return preload_step_sparse_aa_impl<T, true>(peers, resid);
-    if (storage == LBM_STORE_SPARSE_AB) return preload_step_sparse_impl<T, true>(resid);
-    return preload_step_dense_impl<T, true>(storage, speculative, resid);
+    if (storage == LBM_STORE_SPARSE_AA) return preload_step_sparse_aa_impl<T, true, LBM_COLL_BGK>(peers, resid);
+    if (storage == LBM_STORE_SPARSE_AB) return preload_step_sparse_impl<T, true, LBM_COLL_BGK>(resid);
+    return preload_step_dense_impl<T, true, LBM_COLL_BGK>(storage, speculative, resid);
 }
 template cudaError_t preload_step_kernels_strict<float>(int, bool, bool, bool);
 template cudaError_t preload_step_kernels_strict<double>(int, bool, bool, bool);

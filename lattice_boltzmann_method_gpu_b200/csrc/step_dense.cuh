@@ -1,4 +1,4 @@
-// Fused pull-stream + BGK-collide + moment kernel on the box-dense SoA layout,
+// Fused pull-stream + collide (BGK or TRT, lattice.cuh) + moment kernel on the box-dense SoA layout,
 // with link-wise boundaries evaluated by the FLUID node ("fluid-side push").
 //
 // Replaces the reference's `update` + `boundary_stream` pair
@@ -108,7 +108,7 @@ enum { MODE_AB = 0, MODE_AA_EVEN = 1, MODE_AA_ODD = 2 };
 // per NODE in three phases -- all source labels, then all prescribed speeds, then the arithmetic --
 // so that the dependent loads of the links overlap instead of queueing up link after link: these
 // few nodes set the lifetime of their CTA, which is what a small grid's step time consists of.
-template <typename T>
+template <typename T, int COLL>
 __device__ __noinline__ uint32_t boundary_node(const StepParams<T> &p, long long c, uint32_t rest, int mode, T rho, T ux,
                                                T uy, T uz, const T *g, const T *fpre, T *out, T pulse) {
     const Box &b = p.box;
@@ -151,6 +151,8 @@ __device__ __noinline__ uint32_t boundary_node(const StepParams<T> &p, long long
             wm |= 1u << q;
         } else if (bcm & (1u << q)) {
             // feq_q(rho_bc, u_bc(s)) + (g_q(x) - feq_q(rho_x, u_x)) (1 - 1/tau)      (bif:877-1021)
+            // TRT: the extrapolated non-equilibrium n_q = g_q(x) - feq_q(rho_x, u_x) relaxes like the collision,
+            //      feq_q(rho_bc, u_bc(s)) + (1 - om+) (n_q + n_opp(q))/2 + (1 - om-) (n_q - n_opp(q))/2
             const BcEntry &e = p.bc[l];
             const T feq = feq_lit<T>(q, r3, r18, r36, ux, uy, uz);
             T tmp;
@@ -160,7 +162,12 @@ __device__ __noinline__ uint32_t boundary_node(const StepParams<T> &p, long long
                 const T rw = e.kind == LBM_BC_V ? (q < 7 ? r18 : r36) : (q < 7 ? one / T(18.0) : one / T(36.0));
                 tmp = feq_bc_axis<T>(rw, caxis(q, e.vaxis), ubc[q]);
             }
-            out[q] = tmp + (g[q] - feq) * p.om1;
+            if constexpr (COLL == LBM_COLL_TRT) {
+                const T nq = g[q] - feq, nb = g[oppq(q)] - feq_lit<T>(oppq(q), r3, r18, r36, ux, uy, uz);
+                out[q] = tmp + (p.om1 * (T(0.5) * (nq + nb)) + p.om1_m * (T(0.5) * (nq - nb)));
+            } else {
+                out[q] = tmp + (g[q] - feq) * p.om1;
+            }
             wm |= 1u << q;
         } else if (mode != MODE_AB) {
             out[q] = fpre[q];  // static link, in-place storage: the constant travels with the link
@@ -300,7 +307,7 @@ __device__ __forceinline__ void push_to_peers(const StepParams<T> &p, long long 
 
 // WALL_READY: the caller already holds the node's wall mask in `wallw`; otherwise it is fetched here,
 // lazily, by the few nodes that need it
-template <typename T, bool STRICT, bool MOMENTS, bool RESID, int MODE, bool WALL_READY>
+template <typename T, bool STRICT, int COLL, bool MOMENTS, bool RESID, int MODE, bool WALL_READY>
 __device__ __forceinline__ void finish_cell(const StepParams<T> &p, long long c, uint32_t node, uint32_t wallw, T (&f)[Q],
                                             double &velsum) {
     T rho, ux, uy, uz;
@@ -324,7 +331,7 @@ __device__ __forceinline__ void finish_cell(const StepParams<T> &p, long long c,
             for (int q = 0; q < Q; q++) fpre[q] = f[q];
         }
     }
-    collide_bgk<T, STRICT>(f, p.tau, p.inv_tau, rho, ux, uy, uz);
+    collide<T, STRICT, COLL>(f, p, rho, ux, uy, uz);
 #pragma unroll
     for (int q = 0; q < Q; q++) {
         if (MODE == MODE_AA_ODD) {
@@ -366,7 +373,7 @@ __device__ __forceinline__ void finish_cell(const StepParams<T> &p, long long c,
 #pragma unroll
                 for (int q = 0; q < Q; q++) fpre[q] = T(0.0);
             }
-            const uint32_t wm = boundary_node<T>(p, (long long)c, rest, MODE, rho, ux, uy, uz, gl, fpre, hv, p.pulse_scale);
+            const uint32_t wm = boundary_node<T, COLL>(p, (long long)c, rest, MODE, rho, ux, uy, uz, gl, fpre, hv, p.pulse_scale);
 #pragma unroll
             for (int q = 1; q < Q; q++) {
                 if (wm & (1u << q)) {
@@ -389,7 +396,7 @@ __device__ __forceinline__ void grid_dep_wait() { asm volatile("griddepcontrol.w
 // Used by the in-place storages only: the two-buffer kernels read through the non-coherent path (ld.global.nc),
 // whose contract -- read-only for the lifetime of the kernel -- an early-started kernel would break.
 
-template <typename T, bool STRICT, bool MOMENTS, bool RESID, bool SPEC, int CFG, int MODE>
+template <typename T, bool STRICT, int COLL, bool MOMENTS, bool RESID, bool SPEC, int CFG, int MODE>
 __global__ void __launch_bounds__(cfg_block(CFG), cfg_minb(CFG)) k_step_dense(const __grid_constant__ StepParams<T> p) {
     const Box &b = p.box;
     // 64-bit cell ids on purpose: 32-bit ones turn every address into one IMAD.WIDE.U32 instead of an
@@ -436,7 +443,7 @@ __global__ void __launch_bounds__(cfg_block(CFG), cfg_minb(CFG)) k_step_dense(co
                 f[q] = MODE == MODE_AB ? ld_stream(p.pull_base[q] + c) : p.pull_base[q][c];
             }
         }
-        finish_cell<T, STRICT, MOMENTS, RESID, MODE, true>(p, c, node, wallw, f, velsum);
+        finish_cell<T, STRICT, COLL, MOMENTS, RESID, MODE, true>(p, c, node, wallw, f, velsum);
     }
     if (RESID) {
         // warp shuffle tree, then one atomic per warp
@@ -446,7 +453,7 @@ __global__ void __launch_bounds__(cfg_block(CFG), cfg_minb(CFG)) k_step_dense(co
     }
 }
 
-template <typename T, bool STRICT, bool MOMENTS, bool RESID, int CFG, int MODE>
+template <typename T, bool STRICT, int COLL, bool MOMENTS, bool RESID, int CFG, int MODE>
 cudaError_t launch_mode(const StepParams<T> &p, cudaStream_t s) {
     constexpr int B = cfg_block(CFG);
     const unsigned nb = (unsigned)((p.c_end - p.c_begin + B - 1) / B);
@@ -456,18 +463,18 @@ cudaError_t launch_mode(const StepParams<T> &p, cudaStream_t s) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(nb), cfg.blockDim = dim3(B), cfg.dynamicSmemBytes = 0, cfg.stream = s;
     cfg.attrs = at, cfg.numAttrs = (MODE != MODE_AB && p.pdl) ? 1 : 0;
-    if (p.speculative) return cudaLaunchKernelEx(&cfg, k_step_dense<T, STRICT, MOMENTS, RESID, true, CFG, MODE>, p);
-    return cudaLaunchKernelEx(&cfg, k_step_dense<T, STRICT, MOMENTS, RESID, false, CFG, MODE>, p);
+    if (p.speculative) return cudaLaunchKernelEx(&cfg, k_step_dense<T, STRICT, COLL, MOMENTS, RESID, true, CFG, MODE>, p);
+    return cudaLaunchKernelEx(&cfg, k_step_dense<T, STRICT, COLL, MOMENTS, RESID, false, CFG, MODE>, p);
 }
 
-template <typename T, bool STRICT, bool MOMENTS, bool RESID>
+template <typename T, bool STRICT, int COLL, bool MOMENTS, bool RESID>
 cudaError_t launch_cfg(const StepParams<T> &p, int storage, cudaStream_t s) {
     constexpr int C = default_cfg<T>();
     if (storage == LBM_STORE_DENSE_AA) {
-        if (p.parity == 0) return launch_mode<T, STRICT, MOMENTS, RESID, C, MODE_AA_EVEN>(p, s);
-        return launch_mode<T, STRICT, MOMENTS, RESID, C, MODE_AA_ODD>(p, s);
+        if (p.parity == 0) return launch_mode<T, STRICT, COLL, MOMENTS, RESID, C, MODE_AA_EVEN>(p, s);
+        return launch_mode<T, STRICT, COLL, MOMENTS, RESID, C, MODE_AA_ODD>(p, s);
     }
-    return launch_mode<T, STRICT, MOMENTS, RESID, C, MODE_AB>(p, s);
+    return launch_mode<T, STRICT, COLL, MOMENTS, RESID, C, MODE_AB>(p, s);
 }
 
 // host: fold the storage mode into the per-direction base pointers
@@ -498,9 +505,8 @@ void set_bases(StepParams<T> &p) {
     }
 }
 
-template <typename T, bool STRICT>
-cudaError_t launch_step_dense_impl(const StepParams<T> &p_in, bool moments, bool resid, int storage, cudaStream_t s) {
-    if (p_in.c_end <= p_in.c_begin) return cudaSuccess;
+template <typename T, bool STRICT, int COLL>
+cudaError_t launch_step_dense_coll(const StepParams<T> &p_in, bool moments, bool resid, int storage, cudaStream_t s) {
     StepParams<T> p = p_in;
     if (storage == LBM_STORE_DENSE_AA) {
         if (p.parity == 0) set_bases<T, MODE_AA_EVEN>(p);
@@ -508,10 +514,20 @@ cudaError_t launch_step_dense_impl(const StepParams<T> &p_in, bool moments, bool
     } else {
         set_bases<T, MODE_AB>(p);
     }
-    if (moments && resid) return launch_cfg<T, STRICT, true, true>(p, storage, s);
-    if (moments) return launch_cfg<T, STRICT, true, false>(p, storage, s);
-    if (resid) return launch_cfg<T, STRICT, false, true>(p, storage, s);
-    return launch_cfg<T, STRICT, false, false>(p, storage, s);
+    if (moments && resid) return launch_cfg<T, STRICT, COLL, true, true>(p, storage, s);
+    if (moments) return launch_cfg<T, STRICT, COLL, true, false>(p, storage, s);
+    if (resid) return launch_cfg<T, STRICT, COLL, false, true>(p, storage, s);
+    return launch_cfg<T, STRICT, COLL, false, false>(p, storage, s);
+}
+// the collision is a template parameter of every step kernel; TRT kernels exist in FAST arithmetic only
+template <typename T, bool STRICT>
+cudaError_t launch_step_dense_impl(const StepParams<T> &p, bool moments, bool resid, int storage, cudaStream_t s) {
+    if (p.c_end <= p.c_begin) return cudaSuccess;
+    if (p.collision == LBM_COLL_BGK) return launch_step_dense_coll<T, STRICT, LBM_COLL_BGK>(p, moments, resid, storage, s);
+    if constexpr (!STRICT) {
+        if (p.collision == LBM_COLL_TRT) return launch_step_dense_coll<T, false, LBM_COLL_TRT>(p, moments, resid, storage, s);
+    }
+    return cudaErrorInvalidValue;
 }
 
 // With lazy module loading (the CUDA default) a kernel is loaded the first time it is launched -- 5 to 10 ms
@@ -523,29 +539,29 @@ inline cudaError_t preload_kernel(K kernel) {
     cudaFuncAttributes a;
     return cudaFuncGetAttributes(&a, kernel);
 }
-template <typename T, bool STRICT, bool SPEC, int MODE>
+template <typename T, bool STRICT, int COLL, bool SPEC, int MODE>
 cudaError_t preload_dense_mode(bool resid) {  // with and without moments
     constexpr int C = default_cfg<T>();
     cudaError_t e;
     if (resid) {
-        if ((e = preload_kernel(k_step_dense<T, STRICT, false, true, SPEC, C, MODE>)) != cudaSuccess) return e;
-        return preload_kernel(k_step_dense<T, STRICT, true, true, SPEC, C, MODE>);
+        if ((e = preload_kernel(k_step_dense<T, STRICT, COLL, false, true, SPEC, C, MODE>)) != cudaSuccess) return e;
+        return preload_kernel(k_step_dense<T, STRICT, COLL, true, true, SPEC, C, MODE>);
     }
-    if ((e = preload_kernel(k_step_dense<T, STRICT, false, false, SPEC, C, MODE>)) != cudaSuccess) return e;
-    return preload_kernel(k_step_dense<T, STRICT, true, false, SPEC, C, MODE>);
+    if ((e = preload_kernel(k_step_dense<T, STRICT, COLL, false, false, SPEC, C, MODE>)) != cudaSuccess) return e;
+    return preload_kernel(k_step_dense<T, STRICT, COLL, true, false, SPEC, C, MODE>);
 }
-template <typename T, bool STRICT>
+template <typename T, bool STRICT, int COLL>
 cudaError_t preload_step_dense_impl(int storage, bool speculative, bool resid) {
     cudaError_t e;
     if (storage == LBM_STORE_DENSE_AA) {
         if (speculative) {
-            if ((e = preload_dense_mode<T, STRICT, true, MODE_AA_EVEN>(resid)) != cudaSuccess) return e;
-            return preload_dense_mode<T, STRICT, true, MODE_AA_ODD>(resid);
+            if ((e = preload_dense_mode<T, STRICT, COLL, true, MODE_AA_EVEN>(resid)) != cudaSuccess) return e;
+            return preload_dense_mode<T, STRICT, COLL, true, MODE_AA_ODD>(resid);
         }
-        if ((e = preload_dense_mode<T, STRICT, false, MODE_AA_EVEN>(resid)) != cudaSuccess) return e;
-        return preload_dense_mode<T, STRICT, false, MODE_AA_ODD>(resid);
+        if ((e = preload_dense_mode<T, STRICT, COLL, false, MODE_AA_EVEN>(resid)) != cudaSuccess) return e;
+        return preload_dense_mode<T, STRICT, COLL, false, MODE_AA_ODD>(resid);
     }
-    return speculative ? preload_dense_mode<T, STRICT, true, MODE_AB>(resid) : preload_dense_mode<T, STRICT, false, MODE_AB>(resid);
+    return speculative ? preload_dense_mode<T, STRICT, COLL, true, MODE_AB>(resid) : preload_dense_mode<T, STRICT, COLL, false, MODE_AB>(resid);
 }
 
 }  // namespace lbm

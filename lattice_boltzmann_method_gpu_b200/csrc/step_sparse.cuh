@@ -26,7 +26,7 @@ constexpr int SPARSE_BLOCK = 128;
 #define LBM_SP32_MINB 10
 #endif
 
-template <typename T, bool STRICT, bool MOMENTS, bool RESID>
+template <typename T, bool STRICT, int COLL, bool MOMENTS, bool RESID>
 __global__ void __launch_bounds__(SPARSE_BLOCK, sizeof(T) == 8 ? LBM_SP64_MINB : LBM_SP32_MINB)
     k_step_sparse(const __grid_constant__ SparseParams<T> sp) {
     const StepParams<T> &p = sp.base;
@@ -85,7 +85,7 @@ __global__ void __launch_bounds__(SPARSE_BLOCK, sizeof(T) == 8 ? LBM_SP64_MINB :
         }
         T rho, ux, uy, uz;
         if (active) {
-            collide_bgk<T, STRICT>(f, p.tau, p.inv_tau, rho, ux, uy, uz);
+            collide<T, STRICT, COLL>(f, p, rho, ux, uy, uz);
 #pragma unroll
             for (int q = 0; q < Q; q++) {
                 LBM_CHK(p, p.store_base[q] + i);
@@ -113,7 +113,7 @@ __global__ void __launch_bounds__(SPARSE_BLOCK, sizeof(T) == 8 ? LBM_SP64_MINB :
                     T gl[Q], hv[Q];
 #pragma unroll
                     for (int q = 0; q < Q; q++) gl[q] = f[q];
-                    const uint32_t wm = boundary_node<T>(p, c, rest, MODE_AB, rho, ux, uy, uz, gl, gl, hv, p.pulse_scale);
+                    const uint32_t wm = boundary_node<T, COLL>(p, c, rest, MODE_AB, rho, ux, uy, uz, gl, gl, hv, p.pulse_scale);
 #pragma unroll
                     for (int q = 1; q < Q; q++)
                         if (wm & (1u << q)) {
@@ -132,8 +132,8 @@ __global__ void __launch_bounds__(SPARSE_BLOCK, sizeof(T) == 8 ? LBM_SP64_MINB :
     }
 }
 
-template <typename T, bool STRICT>
-cudaError_t launch_step_sparse_impl(const SparseParams<T> &p_in, bool moments, bool resid, cudaStream_t s) {
+template <typename T, bool STRICT, int COLL>
+cudaError_t launch_step_sparse_coll(const SparseParams<T> &p_in, bool moments, bool resid, cudaStream_t s) {
     SparseParams<T> p = p_in;
     for (int q = 0; q < Q; q++) {
         p.base.pull_base[q] = p.base.src + (long long)q * p.base.qstride;
@@ -143,22 +143,30 @@ cudaError_t launch_step_sparse_impl(const SparseParams<T> &p_in, bool moments, b
     if (nrec <= 0) return cudaSuccess;
     const long long n = (nrec + p.spw - 1) / p.spw;  // warps
     const unsigned nb = (unsigned)((n + SPARSE_BLOCK / 32 - 1) / (SPARSE_BLOCK / 32));
-    if (moments && resid) k_step_sparse<T, STRICT, true, true><<<nb, SPARSE_BLOCK, 0, s>>>(p);
-    else if (moments) k_step_sparse<T, STRICT, true, false><<<nb, SPARSE_BLOCK, 0, s>>>(p);
-    else if (resid) k_step_sparse<T, STRICT, false, true><<<nb, SPARSE_BLOCK, 0, s>>>(p);
-    else k_step_sparse<T, STRICT, false, false><<<nb, SPARSE_BLOCK, 0, s>>>(p);
+    if (moments && resid) k_step_sparse<T, STRICT, COLL, true, true><<<nb, SPARSE_BLOCK, 0, s>>>(p);
+    else if (moments) k_step_sparse<T, STRICT, COLL, true, false><<<nb, SPARSE_BLOCK, 0, s>>>(p);
+    else if (resid) k_step_sparse<T, STRICT, COLL, false, true><<<nb, SPARSE_BLOCK, 0, s>>>(p);
+    else k_step_sparse<T, STRICT, COLL, false, false><<<nb, SPARSE_BLOCK, 0, s>>>(p);
     return cudaGetLastError();
 }
-
 template <typename T, bool STRICT>
+cudaError_t launch_step_sparse_impl(const SparseParams<T> &p, bool moments, bool resid, cudaStream_t s) {
+    if (p.base.collision == LBM_COLL_BGK) return launch_step_sparse_coll<T, STRICT, LBM_COLL_BGK>(p, moments, resid, s);
+    if constexpr (!STRICT) {
+        if (p.base.collision == LBM_COLL_TRT) return launch_step_sparse_coll<T, false, LBM_COLL_TRT>(p, moments, resid, s);
+    }
+    return cudaErrorInvalidValue;
+}
+
+template <typename T, bool STRICT, int COLL>
 cudaError_t preload_step_sparse_impl(bool resid) {
     cudaError_t e;
     if (resid) {
-        if ((e = preload_kernel(k_step_sparse<T, STRICT, false, true>)) != cudaSuccess) return e;
-        return preload_kernel(k_step_sparse<T, STRICT, true, true>);
+        if ((e = preload_kernel(k_step_sparse<T, STRICT, COLL, false, true>)) != cudaSuccess) return e;
+        return preload_kernel(k_step_sparse<T, STRICT, COLL, true, true>);
     }
-    if ((e = preload_kernel(k_step_sparse<T, STRICT, false, false>)) != cudaSuccess) return e;
-    return preload_kernel(k_step_sparse<T, STRICT, true, false>);
+    if ((e = preload_kernel(k_step_sparse<T, STRICT, COLL, false, false>)) != cudaSuccess) return e;
+    return preload_kernel(k_step_sparse<T, STRICT, COLL, true, false>);
 }
 
 }  // namespace lbm

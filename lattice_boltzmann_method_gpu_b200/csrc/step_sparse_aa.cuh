@@ -61,11 +61,12 @@ __device__ __forceinline__ T ld_pop(const T *a) {
 
 // inlet / outlet links of a node, after its collision: the non-equilibrium extrapolation value
 //     feq_q(rho_bc, u_bc(s)) + (g_q(x) - feq_q(rho_x, u_x)) (1 - 1/tau)          (bif:877-1021, step_dense.cuh)
+// (under TRT the extrapolated part relaxes with both rates, as in step_dense.cuh boundary_node)
 // goes into the node's own slot.  Which links, of which kind, with which prescribed speed was worked out once
 // by k_bc_links (lbm_geo.cu); here the 18 directions are unrolled with compile-time q, so a boundary node costs
 // a few dozen instructions per link instead of the ~3600-instruction generic path -- on a 64^3 grid the nodes
 // under the lid / at the inlet otherwise set the duration of every step.
-template <typename T>
+template <typename T, int COLL>
 __device__ __forceinline__ void own_slot_bc(const SparseParams<T> &sp, long long i, T rho, T ux, T uy, T uz,
                                             const T (&f)[Q], T pulse) {
     const StepParams<T> &p = sp.base;
@@ -90,7 +91,12 @@ __device__ __forceinline__ void own_slot_bc(const SparseParams<T> &sp, long long
             tmp = feq_bc_axis<T>(rw, cs, u);
         }
         LBM_CHK(p, p.store_base[q] + i);
-        p.store_base[q][i] = tmp + (f[q] - feq) * p.om1;
+        if constexpr (COLL == LBM_COLL_TRT) {  // the rule of step_dense.cuh boundary_node
+            const T nq = f[q] - feq, nb = f[oppq(q)] - feq_lit<T>(oppq(q), r3, r18, r36, ux, uy, uz);
+            p.store_base[q][i] = tmp + (p.om1 * (T(0.5) * (nq + nb)) + p.om1_m * (T(0.5) * (nq - nb)));
+        } else {
+            p.store_base[q][i] = tmp + (f[q] - feq) * p.om1;
+        }
     }
 }
 
@@ -101,7 +107,7 @@ struct AaStep {
 };
 
 // the local (even) step of one node i in [sp.id_begin, sp.id_end)
-template <typename T, bool STRICT, bool PEERS, bool CG>
+template <typename T, bool STRICT, int COLL, bool PEERS, bool CG>
 __device__ __forceinline__ void aa_even_node(const SparseParams<T> &sp, long long i, AaStep st, T pulse, double &velsum) {
     const StepParams<T> &p = sp.base;
     // one word per 32 ids says which lanes are fluid and whether any of them needs its node word at all
@@ -120,7 +126,7 @@ __device__ __forceinline__ void aa_even_node(const SparseParams<T> &sp, long lon
     }
     if ((node & NODE_LINKS) && !(node & NODE_WALLS_ONLY)) rest = node & NODE_LINKS & ~sp.wallc[i];
     T rho, ux, uy, uz;
-    collide_bgk<T, STRICT>(f, p.tau, p.inv_tau, rho, ux, uy, uz);
+    collide<T, STRICT, COLL>(f, p, rho, ux, uy, uz);
     if (rest == 0u) {
 #pragma unroll
         for (int q = 0; q < Q; q++) {
@@ -134,7 +140,7 @@ __device__ __forceinline__ void aa_even_node(const SparseParams<T> &sp, long lon
                 LBM_CHK(p, p.store_base[q] + i);
                 p.store_base[q][i] = f[oppq(q)];
             }
-        if (node & NODE_HAS_BC) own_slot_bc<T>(sp, i, rho, ux, uy, uz, f, pulse);
+        if (node & NODE_HAS_BC) own_slot_bc<T, COLL>(sp, i, rho, ux, uy, uz, f, pulse);
     }
     if (st.moments) {
         p.rho[i] = rho, p.ux[i] = ux, p.uy[i] = uy, p.uz[i] = uz;
@@ -144,7 +150,7 @@ __device__ __forceinline__ void aa_even_node(const SparseParams<T> &sp, long lon
 }
 
 // the neighbour (odd) step of one record: a whole warp calls this with the same `seg`
-template <typename T, bool STRICT, bool PEERS, bool CG>
+template <typename T, bool STRICT, int COLL, bool PEERS, bool CG>
 __device__ __forceinline__ void aa_odd_record(const SparseParams<T> &sp, long long seg, AaStep st, T pulse, double &velsum) {
     const StepParams<T> &p = sp.base;
     const int lane = threadIdx.x & 31;
@@ -188,7 +194,7 @@ __device__ __forceinline__ void aa_odd_record(const SparseParams<T> &sp, long lo
     uint32_t rest = 0u;
     if ((node & NODE_LINKS) && !(node & NODE_WALLS_ONLY)) rest = node & NODE_LINKS & ~sp.wallc[i];
     T rho, ux, uy, uz;
-    collide_bgk<T, STRICT>(f, p.tau, p.inv_tau, rho, ux, uy, uz);
+    collide<T, STRICT, COLL>(f, p, rho, ux, uy, uz);
     LBM_CHK(p, p.store_base[0] + i);
     p.store_base[0][i] = f[0];
 #pragma unroll
@@ -208,7 +214,7 @@ __device__ __forceinline__ void aa_odd_record(const SparseParams<T> &sp, long lo
         LBM_CHK(p, p.store_base[oppq(k)] + idx[k]);
         p.store_base[oppq(k)][idx[k]] = f[oppq(k)];
     }
-    if (rest && (node & NODE_HAS_BC)) own_slot_bc<T>(sp, i, rho, ux, uy, uz, f, pulse);
+    if (rest && (node & NODE_HAS_BC)) own_slot_bc<T, COLL>(sp, i, rho, ux, uy, uz, f, pulse);
     if (st.moments) {
         p.rho[i] = rho, p.ux[i] = ux, p.uy[i] = uy, p.uz[i] = uz;
     }
@@ -232,24 +238,24 @@ __device__ __forceinline__ void cta_add(double *dst, double v) {
     }
 }
 
-template <typename T, bool STRICT, bool MOMENTS, bool RESID, bool PEERS>
+template <typename T, bool STRICT, int COLL, bool MOMENTS, bool RESID, bool PEERS>
 __global__ void __launch_bounds__(SPARSE_BLOCK, sizeof(T) == 8 ? LBM_SPAA64_MINB : LBM_SPAA32_MINB)
     k_sparse_aa_even(const __grid_constant__ SparseParams<T> sp) {
     grid_dep_launch();
     const long long i = sp.id_begin + (long long)blockIdx.x * SPARSE_BLOCK + threadIdx.x;
     double velsum = 0.0;
-    aa_even_node<T, STRICT, PEERS, false>(sp, i, AaStep{MOMENTS, RESID}, sp.base.pulse_scale, velsum);
+    aa_even_node<T, STRICT, COLL, PEERS, false>(sp, i, AaStep{MOMENTS, RESID}, sp.base.pulse_scale, velsum);
     if (RESID) cta_add<SPARSE_BLOCK / 32>(sp.base.resid, velsum);
 }
 
-template <typename T, bool STRICT, bool MOMENTS, bool RESID, bool PEERS>
+template <typename T, bool STRICT, int COLL, bool MOMENTS, bool RESID, bool PEERS>
 __global__ void __launch_bounds__(SPARSE_BLOCK, sizeof(T) == 8 ? LBM_SPAA64_ODD_MINB : LBM_SPAA32_ODD_MINB)
     k_sparse_aa_odd(const __grid_constant__ SparseParams<T> sp) {
     grid_dep_launch();
     const long long seg = sp.seg_begin + (long long)blockIdx.x * (SPARSE_BLOCK / 32) + (threadIdx.x >> 5);
     double velsum = 0.0;
     if (seg < sp.seg_end)  // warp-uniform
-        aa_odd_record<T, STRICT, PEERS, false>(sp, seg, AaStep{MOMENTS, RESID}, sp.base.pulse_scale, velsum);
+        aa_odd_record<T, STRICT, COLL, PEERS, false>(sp, seg, AaStep{MOMENTS, RESID}, sp.base.pulse_scale, velsum);
     if (RESID) cta_add<SPARSE_BLOCK / 32>(sp.base.resid, velsum);
 }
 
@@ -300,7 +306,7 @@ __device__ __forceinline__ void grid_barrier(unsigned *bar, unsigned gen) {
 // 1480 CTAs of 128 threads made a step 19 us, one or two CTAs of 512 threads per SM keep it near the L2
 // round trip (profiles/r02_notes.md).
 constexpr int PERSIST_BLOCK = 512;
-template <typename T, bool STRICT>
+template <typename T, bool STRICT, int COLL>
 __global__ void __launch_bounds__(PERSIST_BLOCK, sizeof(T) == 8 ? 1 : 2)
     k_sparse_aa_persist(const __grid_constant__ SparseParams<T> sp, const __grid_constant__ PersistArgs<T> pa) {
     const long long warp0 = (long long)blockIdx.x * (PERSIST_BLOCK / 32) + (threadIdx.x >> 5);
@@ -314,18 +320,18 @@ __global__ void __launch_bounds__(PERSIST_BLOCK, sizeof(T) == 8 ? 1 : 2)
         if (((pa.parity0 + s) & 1) == 0) {
             for (long long c = first_chunk + warp0; c < end_chunk; c += nwarps) {
                 const long long i = c * 32 + lane;
-                if (i >= sp.id_begin) aa_even_node<T, STRICT, false, true>(sp, i, st, pulse, velsum);
+                if (i >= sp.id_begin) aa_even_node<T, STRICT, COLL, false, true>(sp, i, st, pulse, velsum);
             }
         } else {
             for (long long seg = sp.seg_begin + warp0; seg < sp.seg_end; seg += nwarps)
-                aa_odd_record<T, STRICT, false, true>(sp, seg, st, pulse, velsum);
+                aa_odd_record<T, STRICT, COLL, false, true>(sp, seg, st, pulse, velsum);
         }
         if (st.resid) cta_add<PERSIST_BLOCK / 32>(pa.S + s, velsum);
         if (s + 1 < pa.nsteps) grid_barrier(pa.barrier, (unsigned)(s + 1));
     }
 }
-template <typename T, bool STRICT>
-cudaError_t launch_sparse_aa_persist_impl(const SparseParams<T> &p_in, const PersistArgs<T> &pa, int sm_count, cudaStream_t s) {
+template <typename T, bool STRICT, int COLL>
+cudaError_t launch_sparse_aa_persist_coll(const SparseParams<T> &p_in, const PersistArgs<T> &pa, int sm_count, cudaStream_t s) {
     SparseParams<T> p = p_in;
     for (int q = 0; q < Q; q++) {
         p.base.pull_base[q] = p.base.src + (long long)q * p.base.qstride;
@@ -333,7 +339,7 @@ cudaError_t launch_sparse_aa_persist_impl(const SparseParams<T> &p_in, const Per
         p.dk[q] = (int)((long long)(q - oppq(q)) * p.base.qstride);
     }
     int per_sm = 0;
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sparse_aa_persist<T, STRICT>, PERSIST_BLOCK, 0);
+    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sparse_aa_persist<T, STRICT, COLL>, PERSIST_BLOCK, 0);
     if (e != cudaSuccess) return e;
     if (per_sm < 1) return cudaErrorLaunchOutOfResources;
     per_sm = std::min(per_sm, sizeof(T) == 8 ? 1 : 2);
@@ -345,10 +351,18 @@ cudaError_t launch_sparse_aa_persist_impl(const SparseParams<T> &p_in, const Per
     long long blocks = std::max<long long>(1, std::min(max_blocks, (warps + wpb - 1) / wpb));
     PersistArgs<T> a = pa;
     void *args[2] = {(void *)&p, (void *)&a};
-    return cudaLaunchCooperativeKernel((const void *)k_sparse_aa_persist<T, STRICT>, dim3((unsigned)blocks), dim3(PERSIST_BLOCK), args, 0, s);
+    return cudaLaunchCooperativeKernel((const void *)k_sparse_aa_persist<T, STRICT, COLL>, dim3((unsigned)blocks), dim3(PERSIST_BLOCK), args, 0, s);
+}
+template <typename T, bool STRICT>
+cudaError_t launch_sparse_aa_persist_impl(const SparseParams<T> &p, const PersistArgs<T> &pa, int sm_count, cudaStream_t s) {
+    if (p.base.collision == LBM_COLL_BGK) return launch_sparse_aa_persist_coll<T, STRICT, LBM_COLL_BGK>(p, pa, sm_count, s);
+    if constexpr (!STRICT) {
+        if (p.base.collision == LBM_COLL_TRT) return launch_sparse_aa_persist_coll<T, false, LBM_COLL_TRT>(p, pa, sm_count, s);
+    }
+    return cudaErrorInvalidValue;
 }
 
-template <typename T, bool STRICT, bool MOMENTS, bool RESID, bool PEERS>
+template <typename T, bool STRICT, int COLL, bool MOMENTS, bool RESID, bool PEERS>
 cudaError_t launch_sparse_aa_mode(const SparseParams<T> &p, cudaStream_t s) {
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -360,17 +374,17 @@ cudaError_t launch_sparse_aa_mode(const SparseParams<T> &p, cudaStream_t s) {
         const long long n = p.id_end - p.id_begin;
         if (n <= 0) return cudaSuccess;
         cfg.gridDim = dim3((unsigned)((n + SPARSE_BLOCK - 1) / SPARSE_BLOCK));
-        return cudaLaunchKernelEx(&cfg, k_sparse_aa_even<T, STRICT, MOMENTS, RESID, PEERS>, p);
+        return cudaLaunchKernelEx(&cfg, k_sparse_aa_even<T, STRICT, COLL, MOMENTS, RESID, PEERS>, p);
     }
     const long long nrec = p.seg_end - p.seg_begin;
     if (nrec <= 0) return cudaSuccess;
     const int wpb = SPARSE_BLOCK / 32;
     cfg.gridDim = dim3((unsigned)((nrec + wpb - 1) / wpb));
-    return cudaLaunchKernelEx(&cfg, k_sparse_aa_odd<T, STRICT, MOMENTS, RESID, PEERS>, p);
+    return cudaLaunchKernelEx(&cfg, k_sparse_aa_odd<T, STRICT, COLL, MOMENTS, RESID, PEERS>, p);
 }
 
-template <typename T, bool STRICT>
-cudaError_t launch_step_sparse_aa_impl(const SparseParams<T> &p_in, bool moments, bool resid, cudaStream_t s) {
+template <typename T, bool STRICT, int COLL>
+cudaError_t launch_step_sparse_aa_coll(const SparseParams<T> &p_in, bool moments, bool resid, cudaStream_t s) {
     SparseParams<T> p = p_in;
     for (int q = 0; q < Q; q++) {
         p.base.pull_base[q] = p.base.src + (long long)q * p.base.qstride;
@@ -379,20 +393,28 @@ cudaError_t launch_step_sparse_aa_impl(const SparseParams<T> &p_in, bool moments
     }
     const bool peers = p.base.peer_up || p.base.peer_dn;
 #define LBM_SPAA(M, R)                                                                    \
-    (peers ? launch_sparse_aa_mode<T, STRICT, M, R, true>(p, s) : launch_sparse_aa_mode<T, STRICT, M, R, false>(p, s))
+    (peers ? launch_sparse_aa_mode<T, STRICT, COLL, M, R, true>(p, s) : launch_sparse_aa_mode<T, STRICT, COLL, M, R, false>(p, s))
     if (moments && resid) return LBM_SPAA(true, true);
     if (moments) return LBM_SPAA(true, false);
     if (resid) return LBM_SPAA(false, true);
     return LBM_SPAA(false, false);
 #undef LBM_SPAA
 }
+template <typename T, bool STRICT>
+cudaError_t launch_step_sparse_aa_impl(const SparseParams<T> &p, bool moments, bool resid, cudaStream_t s) {
+    if (p.base.collision == LBM_COLL_BGK) return launch_step_sparse_aa_coll<T, STRICT, LBM_COLL_BGK>(p, moments, resid, s);
+    if constexpr (!STRICT) {
+        if (p.base.collision == LBM_COLL_TRT) return launch_step_sparse_aa_coll<T, false, LBM_COLL_TRT>(p, moments, resid, s);
+    }
+    return cudaErrorInvalidValue;
+}
 
-template <typename T, bool STRICT, bool PEERS>
+template <typename T, bool STRICT, int COLL, bool PEERS>
 cudaError_t preload_sparse_aa_peers(bool resid) {
     cudaError_t e;
 #define LBM_PL(M, R)                                                                                      \
-    if ((e = preload_kernel(k_sparse_aa_even<T, STRICT, M, R, PEERS>)) != cudaSuccess) return e;          \
-    if ((e = preload_kernel(k_sparse_aa_odd<T, STRICT, M, R, PEERS>)) != cudaSuccess) return e;
+    if ((e = preload_kernel(k_sparse_aa_even<T, STRICT, COLL, M, R, PEERS>)) != cudaSuccess) return e;          \
+    if ((e = preload_kernel(k_sparse_aa_odd<T, STRICT, COLL, M, R, PEERS>)) != cudaSuccess) return e;
     if (resid) {
         LBM_PL(false, true) LBM_PL(true, true)
     } else {
@@ -401,9 +423,9 @@ cudaError_t preload_sparse_aa_peers(bool resid) {
 #undef LBM_PL
     return cudaSuccess;
 }
-template <typename T, bool STRICT>
+template <typename T, bool STRICT, int COLL>
 cudaError_t preload_step_sparse_aa_impl(bool peers, bool resid) {
-    return peers ? preload_sparse_aa_peers<T, STRICT, true>(resid) : preload_sparse_aa_peers<T, STRICT, false>(resid);
+    return peers ? preload_sparse_aa_peers<T, STRICT, COLL, true>(resid) : preload_sparse_aa_peers<T, STRICT, COLL, false>(resid);
 }
 
 }  // namespace lbm
