@@ -20,6 +20,7 @@
 #include <sstream>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "lbm_internal.h"
@@ -742,13 +743,17 @@ struct Solver final : SolverBase {
         static const char *const force = getenv("LBM_SPECULATIVE");  // tuning knob, read once
         return force ? atoi(force) != 0 : (nfluid * 10 >= (int64_t)(own_z1 - own_z0) * box.plane * 9);
     }
+    // f(std::bool_constant<STRICT>) for this handle's arithmetic: the step entry points are instantiated per arithmetic
+    template <typename F>
+    cudaError_t with_math(F f) const {
+        if (d.math == LBM_MATH_STRICT) return f(std::true_type{});
+        return f(std::false_type{});
+    }
     // the run loops load the step kernels they are about to launch before they start their clock (lazy module
-    // loading would otherwise put 5 - 10 ms per kernel variant into the loop: step_dense.cuh preload_kernel)
+    // loading would otherwise put 5 - 10 ms per kernel variant into the loop: step_launch.cuh preload_step_kernels)
     int preload_kernels(bool resid) {
-        const bool peers = lo_halo || hi_halo;
         CK(cudaSetDevice(d.device));
-        if (d.math == LBM_MATH_STRICT) CK(preload_step_kernels_strict<T>(d.storage, speculative_pull(), peers, resid));
-        else CK(preload_step_kernels_fast<T>(d.storage, speculative_pull(), peers, resid, collision));
+        CK(with_math([&](auto S) { return preload_step_kernels<T, S>(d.storage, collision, speculative_pull(), resid, use_persist()); }));
         return 0;
     }
 
@@ -787,40 +792,31 @@ struct Solver final : SolverBase {
         p.speculative = speculative_pull();
         return p;
     }
+    // the parameters of a launch over the cells [c0, c1) of the state box; a sparse storage adds its records and id
+    // ranges, the dense ones use .base only.  face_sides bit 0: the range is the lowest owned plane, bit 1: the highest
+    SparseParams<T> launch_params(long long c0, long long c1, double *acc, int face_sides) {
+        SparseParams<T> sp{};
+        sp.base = make_params(c0, c1, acc);
+        for (int sd = 0; sd < 2; sd++)
+            if (face_sides & (1 << sd)) link_params(sp.base, sd, c0);
+        if (!sparse) return sp;
+        static const int spw_env = getenv("LBM_SPW") ? atoi(getenv("LBM_SPW")) : 0;  // tuning knob
+        sp.spw = spw_env > 0 ? spw_env : 1;  // measured: 1 is fastest (profiles/r01_notes.md)
+        sp.rec = d_rec, sp.nodec = d_nodec, sp.wallc = d_wallc;
+        sp.cartc = d_cart, sp.cmeta = d_cmeta, sp.rec_links = d_rec_links, sp.bcslot = d_bcslot, sp.bclinks = d_bclinks;
+        const long long zA = c0 / box.plane - (own_z0 - box.z0), zB = c1 / box.plane - (own_z0 - box.z0);
+        sp.seg_begin = seg_plane_start[(size_t)zA], sp.seg_end = seg_plane_start[(size_t)zB];
+        sp.id_begin = sid_plane_first[(size_t)(c0 / box.plane)], sp.id_end = sid_plane_first[(size_t)(c1 / box.plane)];
+        sp.halo_lo_n = (int)halo_n[0], sp.halo_hi0 = (int)halo_id0[1];
+        return sp;
+    }
     int launch_range(long long c0, long long c1, bool moments, bool resid, double *acc, int face_sides = 0) {
         if (c1 <= c0) return 0;
-        StepParams<T> p = make_params(c0, c1, acc);
-        // face_sides bit 0: this range is the lowest owned plane, bit 1: the highest
-        for (int sd = 0; sd < 2; sd++)
-            if (face_sides & (1 << sd)) link_params(p, sd, c0);
-        if (sparse) {
-            SparseParams<T> sp{};
-            sp.base = p, sp.rec = d_rec, sp.nodec = d_nodec, sp.wallc = d_wallc;
-            {
-                static const int spw_env = getenv("LBM_SPW") ? atoi(getenv("LBM_SPW")) : 0;  // tuning knob
-                sp.spw = spw_env > 0 ? spw_env : 1;   // measured: 1 is fastest (profiles/r01_notes.md)
-            }
-            const long long zA = c0 / box.plane - (own_z0 - box.z0), zB = c1 / box.plane - (own_z0 - box.z0);
-            sp.seg_begin = seg_plane_start[(size_t)zA], sp.seg_end = seg_plane_start[(size_t)zB];
-            if (d.storage == LBM_STORE_SPARSE_AA) {
-                sp.cartc = d_cart, sp.cmeta = d_cmeta, sp.rec_links = d_rec_links, sp.bcslot = d_bcslot, sp.bclinks = d_bclinks;
-                sp.id_begin = sid_plane_first[(size_t)(c0 / box.plane)], sp.id_end = sid_plane_first[(size_t)(c1 / box.plane)];
-                sp.halo_lo_n = (int)halo_n[0], sp.halo_hi0 = (int)halo_id0[1];
-                sp.pdl = sp.base.pdl;
-                if (sp.base.parity == 0 ? sp.id_end <= sp.id_begin : sp.seg_end <= sp.seg_begin) return 0;
-                if (d.math == LBM_MATH_STRICT) CK(launch_step_sparse_aa_strict<T>(sp, moments, resid, st));
-                else CK(launch_step_sparse_aa_fast<T>(sp, moments, resid, st));
-                launches++;
-                return 0;
-            }
-            if (sp.seg_end <= sp.seg_begin) return 0;
-            if (d.math == LBM_MATH_STRICT) CK(launch_step_sparse_strict<T>(sp, moments, resid, st));
-            else CK(launch_step_sparse_fast<T>(sp, moments, resid, st));
-            launches++;
-            return 0;
-        }
-        if (d.math == LBM_MATH_STRICT) CK(launch_step_dense_strict<T>(p, moments, resid, d.storage, st));
-        else CK(launch_step_dense_fast<T>(p, moments, resid, d.storage, st));
+        const SparseParams<T> sp = launch_params(c0, c1, acc, face_sides);
+        // a sparse kernel walks records (ids on even steps of the in-place storage): planes without fluid have none
+        const bool walks_ids = d.storage == LBM_STORE_SPARSE_AA && sp.base.parity == 0;
+        if (sparse && (walks_ids ? sp.id_end <= sp.id_begin : sp.seg_end <= sp.seg_begin)) return 0;
+        CK(with_math([&](auto S) { return launch_step<T, S>(sp, d.storage, moments, resid, st); }));
         launches++;
         return 0;
     }
@@ -869,16 +865,11 @@ struct Solver final : SolverBase {
             pulse_dev = d_pulse;
         }
         CK(cudaMemsetAsync(d_barrier, 0, PERSIST_BAR_WORDS * sizeof(unsigned), st));
-        SparseParams<T> sp{};
-        sp.base = make_params(plane_c(own_z0), plane_c(own_z1), nullptr);
-        sp.rec = d_rec, sp.nodec = d_nodec, sp.wallc = d_wallc, sp.spw = 1, sp.cartc = d_cart, sp.cmeta = d_cmeta, sp.rec_links = d_rec_links;
-        sp.bcslot = d_bcslot, sp.bclinks = d_bclinks;
-        sp.seg_begin = seg_plane_start[0], sp.seg_end = seg_plane_start[(size_t)(own_z1 - own_z0)];
-        sp.id_begin = own_id0, sp.id_end = own_id1;
-        sp.halo_lo_n = 0, sp.halo_hi0 = INT32_MAX;
+        const SparseParams<T> sp = launch_params(plane_c(own_z0), plane_c(own_z1), nullptr, 0);
         const int parity0 = (int)(steps & 1);
-        if (d.math == LBM_MATH_STRICT) CK(launch_sparse_aa_persist_strict<T>(sp, n, parity0, moments_last ? 1 : 0, S_dev, pulse_dev, d_barrier, sm_count, st));
-        else CK(launch_sparse_aa_persist_fast<T>(sp, n, parity0, moments_last ? 1 : 0, S_dev, pulse_dev, d_barrier, sm_count, st));
+        CK(with_math([&](auto S) {
+            return launch_persist<T, S>(sp, n, parity0, moments_last ? 1 : 0, S_dev, pulse_dev, d_barrier, sm_count, st);
+        }));
         launches++;
         steps += n;
         return 0;

@@ -88,7 +88,7 @@ struct StepParams {
     T *mail[2];                     // this slab's own mailboxes (low / high side) when the launch covers that face, else null
     long long mail_ms, mail_G;
     int peer_mail;                  // peer_up / peer_dn point at the neighbour's mailbox (part A on even, part B on odd steps)
-    int pdl;                        // in-place storages: launch with programmatic stream serialization (step_dense.cuh)
+    int pdl;                        // in-place storages: launch with programmatic stream serialization (step_launch.cuh)
     // per-direction base pointers of the dense kernels, so that an access is base[q] + c (one 64-bit
     // add) instead of five integer instructions: pull_base[q][c] is the population direction q pulls
     // for cell c, store_base[q][c] the slot its post-collision value goes to (storage mode folded in)
@@ -250,32 +250,18 @@ struct SparseParams {
     long long id_begin, id_end;  // compact ids of the even (local) step's launch
     int halo_lo_n, halo_hi0;     // local ids < halo_lo_n lie in the low halo plane, ids >= halo_hi0 in the high one
     int dk[Q];                   // (k - opp k) * qstride: from the array of opp(k) to the same node's slot in the array of k
-    int pdl;                     // launch with programmatic stream serialization (step_sparse_aa.cuh)
 };
 
-// fused step (lbm_step_fast.cu / lbm_step_strict.cu)
-template <typename T>
-cudaError_t launch_step_sparse_fast(const SparseParams<T> &p, bool moments, bool resid, cudaStream_t s);
-template <typename T>
-cudaError_t launch_step_sparse_strict(const SparseParams<T> &p, bool moments, bool resid, cudaStream_t s);
-template <typename T>
-cudaError_t launch_step_sparse_aa_fast(const SparseParams<T> &p, bool moments, bool resid, cudaStream_t s);
-template <typename T>
-cudaError_t launch_step_sparse_aa_strict(const SparseParams<T> &p, bool moments, bool resid, cudaStream_t s);
-template <typename T>
-cudaError_t preload_step_kernels_fast(int storage, bool speculative, bool peers, bool resid, int collision);
-template <typename T>
-cudaError_t preload_step_kernels_strict(int storage, bool speculative, bool peers, bool resid);
+// fused step (step_launch.cuh), instantiated for STRICT = false in lbm_step_fast.cu and true in lbm_step_strict.cu
+// one step over the range of sp, which the caller checked is not empty; the dense storages read sp.base only
+template <typename T, bool STRICT>
+cudaError_t launch_step(const SparseParams<T> &sp, int storage, bool moments, bool resid, cudaStream_t s);
 // nsteps steps of a single-domain in-place sparse handle in ONE cooperative launch (grids that live in L2)
-template <typename T>
-cudaError_t launch_sparse_aa_persist_fast(const SparseParams<T> &p, int nsteps, int parity0, int moments_last, double *S,
-                                          const T *pulse, unsigned *barrier, int sm_count, cudaStream_t s);
-template <typename T>
-cudaError_t launch_sparse_aa_persist_strict(const SparseParams<T> &p, int nsteps, int parity0, int moments_last, double *S,
-                                            const T *pulse, unsigned *barrier, int sm_count, cudaStream_t s);
-template <typename T>
-cudaError_t launch_step_dense_fast(const StepParams<T> &p, bool moments, bool resid, int storage, cudaStream_t s);
-template <typename T>
-cudaError_t launch_step_dense_strict(const StepParams<T> &p, bool moments, bool resid, int storage, cudaStream_t s);
+template <typename T, bool STRICT>
+cudaError_t launch_persist(const SparseParams<T> &sp, int nsteps, int parity0, int moments_last, double *S, const T *pulse,
+                           unsigned *barrier, int sm_count, cudaStream_t s);
+// loads the step kernels a run loop is about to launch
+template <typename T, bool STRICT>
+cudaError_t preload_step_kernels(int storage, int collision, bool speculative, bool resid, bool persist);
 
 }  // namespace lbm

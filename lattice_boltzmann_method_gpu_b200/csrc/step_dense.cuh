@@ -193,24 +193,13 @@ __device__ __noinline__ uint32_t boundary_node(const StepParams<T> &p, long long
 // anything else: CTA shape and register cap are picked per precision
 // (fp64: 128 threads x 6 CTAs/SM, 80 registers; fp32: 128 x 10, 48 registers; no spills).
 // Measurements behind every choice here: profiles/r01_notes.md.
-__host__ __device__ constexpr int cfg_block(int cfg) {
-    constexpr int b[4] = {256, 256, 128, 128};
-    return b[cfg];
-}
+constexpr int DENSE_BLOCK = 128;
 #ifndef LBM_F32_MINB
 #define LBM_F32_MINB 10
 #endif
 #ifndef LBM_F64_MINB
 #define LBM_F64_MINB 6
 #endif
-__host__ __device__ constexpr int cfg_minb(int cfg) {
-    constexpr int m[4] = {2, 3, LBM_F64_MINB, LBM_F32_MINB};
-    return m[cfg];
-}
-template <typename T>
-constexpr int default_cfg() {
-    return sizeof(T) == 8 ? 2 : 3;
-}
 
 // Loads of the speculative pull.  They have to be ISSUED before the thread knows whether it needs them, and
 // ptxas sinks an ordinary ld.global (also .nc, also from `asm volatile`) below the early exit that depends on
@@ -396,14 +385,15 @@ __device__ __forceinline__ void grid_dep_wait() { asm volatile("griddepcontrol.w
 // Used by the in-place storages only: the two-buffer kernels read through the non-coherent path (ld.global.nc),
 // whose contract -- read-only for the lifetime of the kernel -- an early-started kernel would break.
 
-template <typename T, bool STRICT, int COLL, bool MOMENTS, bool RESID, bool SPEC, int CFG, int MODE>
-__global__ void __launch_bounds__(cfg_block(CFG), cfg_minb(CFG)) k_step_dense(const __grid_constant__ StepParams<T> p) {
+template <typename T, bool STRICT, int COLL, bool MOMENTS, bool RESID, bool SPEC, int MODE>
+__global__ void __launch_bounds__(DENSE_BLOCK, sizeof(T) == 8 ? LBM_F64_MINB : LBM_F32_MINB)
+    k_step_dense(const __grid_constant__ StepParams<T> p) {
     const Box &b = p.box;
     // 64-bit cell ids on purpose: 32-bit ones turn every address into one IMAD.WIDE.U32 instead of an
     // IADD3 pair (-22 instructions per thread), which changes nothing in fp64 and costs 6 % in fp32,
     // where IMAD shares its pipe with the collision's FFMAs (profiles/r01_notes.md)
     if (MODE != MODE_AB) grid_dep_launch();
-    const long long c = p.c_begin + (long long)blockIdx.x * cfg_block(CFG) + threadIdx.x;
+    const long long c = p.c_begin + (long long)blockIdx.x * DENSE_BLOCK + threadIdx.x;
     if (c >= p.c_end) return;  // ranges are whole planes (multiples of 32 cells): warp-uniform
     T f[Q];
     uint32_t node, wallw = 0u;
@@ -453,30 +443,6 @@ __global__ void __launch_bounds__(cfg_block(CFG), cfg_minb(CFG)) k_step_dense(co
     }
 }
 
-template <typename T, bool STRICT, int COLL, bool MOMENTS, bool RESID, int CFG, int MODE>
-cudaError_t launch_mode(const StepParams<T> &p, cudaStream_t s) {
-    constexpr int B = cfg_block(CFG);
-    const unsigned nb = (unsigned)((p.c_end - p.c_begin + B - 1) / B);
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(nb), cfg.blockDim = dim3(B), cfg.dynamicSmemBytes = 0, cfg.stream = s;
-    cfg.attrs = at, cfg.numAttrs = (MODE != MODE_AB && p.pdl) ? 1 : 0;
-    if (p.speculative) return cudaLaunchKernelEx(&cfg, k_step_dense<T, STRICT, COLL, MOMENTS, RESID, true, CFG, MODE>, p);
-    return cudaLaunchKernelEx(&cfg, k_step_dense<T, STRICT, COLL, MOMENTS, RESID, false, CFG, MODE>, p);
-}
-
-template <typename T, bool STRICT, int COLL, bool MOMENTS, bool RESID>
-cudaError_t launch_cfg(const StepParams<T> &p, int storage, cudaStream_t s) {
-    constexpr int C = default_cfg<T>();
-    if (storage == LBM_STORE_DENSE_AA) {
-        if (p.parity == 0) return launch_mode<T, STRICT, COLL, MOMENTS, RESID, C, MODE_AA_EVEN>(p, s);
-        return launch_mode<T, STRICT, COLL, MOMENTS, RESID, C, MODE_AA_ODD>(p, s);
-    }
-    return launch_mode<T, STRICT, COLL, MOMENTS, RESID, C, MODE_AB>(p, s);
-}
-
 // host: fold the storage mode into the per-direction base pointers
 template <typename T, int MODE>
 void set_bases(StepParams<T> &p) {
@@ -503,65 +469,6 @@ void set_bases(StepParams<T> &p) {
             }
         }
     }
-}
-
-template <typename T, bool STRICT, int COLL>
-cudaError_t launch_step_dense_coll(const StepParams<T> &p_in, bool moments, bool resid, int storage, cudaStream_t s) {
-    StepParams<T> p = p_in;
-    if (storage == LBM_STORE_DENSE_AA) {
-        if (p.parity == 0) set_bases<T, MODE_AA_EVEN>(p);
-        else set_bases<T, MODE_AA_ODD>(p);
-    } else {
-        set_bases<T, MODE_AB>(p);
-    }
-    if (moments && resid) return launch_cfg<T, STRICT, COLL, true, true>(p, storage, s);
-    if (moments) return launch_cfg<T, STRICT, COLL, true, false>(p, storage, s);
-    if (resid) return launch_cfg<T, STRICT, COLL, false, true>(p, storage, s);
-    return launch_cfg<T, STRICT, COLL, false, false>(p, storage, s);
-}
-// the collision is a template parameter of every step kernel; TRT kernels exist in FAST arithmetic only
-template <typename T, bool STRICT>
-cudaError_t launch_step_dense_impl(const StepParams<T> &p, bool moments, bool resid, int storage, cudaStream_t s) {
-    if (p.c_end <= p.c_begin) return cudaSuccess;
-    if (p.collision == LBM_COLL_BGK) return launch_step_dense_coll<T, STRICT, LBM_COLL_BGK>(p, moments, resid, storage, s);
-    if constexpr (!STRICT) {
-        if (p.collision == LBM_COLL_TRT) return launch_step_dense_coll<T, false, LBM_COLL_TRT>(p, moments, resid, storage, s);
-    }
-    return cudaErrorInvalidValue;
-}
-
-// With lazy module loading (the CUDA default) a kernel is loaded the first time it is launched -- 5 to 10 ms
-// each for functions of this size, 18 ms of a 65 ms drivers/ldc run.  The run loops (lbm_run_fixed,
-// lbm_run_converge) ask for the attributes of the step kernels they are about to launch before they start their
-// clock, which loads them; lbm_step keeps the lazy behaviour (it would load variants it may never use).
-template <typename K>
-inline cudaError_t preload_kernel(K kernel) {
-    cudaFuncAttributes a;
-    return cudaFuncGetAttributes(&a, kernel);
-}
-template <typename T, bool STRICT, int COLL, bool SPEC, int MODE>
-cudaError_t preload_dense_mode(bool resid) {  // with and without moments
-    constexpr int C = default_cfg<T>();
-    cudaError_t e;
-    if (resid) {
-        if ((e = preload_kernel(k_step_dense<T, STRICT, COLL, false, true, SPEC, C, MODE>)) != cudaSuccess) return e;
-        return preload_kernel(k_step_dense<T, STRICT, COLL, true, true, SPEC, C, MODE>);
-    }
-    if ((e = preload_kernel(k_step_dense<T, STRICT, COLL, false, false, SPEC, C, MODE>)) != cudaSuccess) return e;
-    return preload_kernel(k_step_dense<T, STRICT, COLL, true, false, SPEC, C, MODE>);
-}
-template <typename T, bool STRICT, int COLL>
-cudaError_t preload_step_dense_impl(int storage, bool speculative, bool resid) {
-    cudaError_t e;
-    if (storage == LBM_STORE_DENSE_AA) {
-        if (speculative) {
-            if ((e = preload_dense_mode<T, STRICT, COLL, true, MODE_AA_EVEN>(resid)) != cudaSuccess) return e;
-            return preload_dense_mode<T, STRICT, COLL, true, MODE_AA_ODD>(resid);
-        }
-        if ((e = preload_dense_mode<T, STRICT, COLL, false, MODE_AA_EVEN>(resid)) != cudaSuccess) return e;
-        return preload_dense_mode<T, STRICT, COLL, false, MODE_AA_ODD>(resid);
-    }
-    return speculative ? preload_dense_mode<T, STRICT, COLL, true, MODE_AB>(resid) : preload_dense_mode<T, STRICT, COLL, false, MODE_AB>(resid);
 }
 
 }  // namespace lbm

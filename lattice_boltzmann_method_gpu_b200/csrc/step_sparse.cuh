@@ -132,41 +132,4 @@ __global__ void __launch_bounds__(SPARSE_BLOCK, sizeof(T) == 8 ? LBM_SP64_MINB :
     }
 }
 
-template <typename T, bool STRICT, int COLL>
-cudaError_t launch_step_sparse_coll(const SparseParams<T> &p_in, bool moments, bool resid, cudaStream_t s) {
-    SparseParams<T> p = p_in;
-    for (int q = 0; q < Q; q++) {
-        p.base.pull_base[q] = p.base.src + (long long)q * p.base.qstride;
-        p.base.store_base[q] = p.base.dst + (long long)q * p.base.qstride;
-    }
-    const long long nrec = p.seg_end - p.seg_begin;
-    if (nrec <= 0) return cudaSuccess;
-    const long long n = (nrec + p.spw - 1) / p.spw;  // warps
-    const unsigned nb = (unsigned)((n + SPARSE_BLOCK / 32 - 1) / (SPARSE_BLOCK / 32));
-    if (moments && resid) k_step_sparse<T, STRICT, COLL, true, true><<<nb, SPARSE_BLOCK, 0, s>>>(p);
-    else if (moments) k_step_sparse<T, STRICT, COLL, true, false><<<nb, SPARSE_BLOCK, 0, s>>>(p);
-    else if (resid) k_step_sparse<T, STRICT, COLL, false, true><<<nb, SPARSE_BLOCK, 0, s>>>(p);
-    else k_step_sparse<T, STRICT, COLL, false, false><<<nb, SPARSE_BLOCK, 0, s>>>(p);
-    return cudaGetLastError();
-}
-template <typename T, bool STRICT>
-cudaError_t launch_step_sparse_impl(const SparseParams<T> &p, bool moments, bool resid, cudaStream_t s) {
-    if (p.base.collision == LBM_COLL_BGK) return launch_step_sparse_coll<T, STRICT, LBM_COLL_BGK>(p, moments, resid, s);
-    if constexpr (!STRICT) {
-        if (p.base.collision == LBM_COLL_TRT) return launch_step_sparse_coll<T, false, LBM_COLL_TRT>(p, moments, resid, s);
-    }
-    return cudaErrorInvalidValue;
-}
-
-template <typename T, bool STRICT, int COLL>
-cudaError_t preload_step_sparse_impl(bool resid) {
-    cudaError_t e;
-    if (resid) {
-        if ((e = preload_kernel(k_step_sparse<T, STRICT, COLL, false, true>)) != cudaSuccess) return e;
-        return preload_kernel(k_step_sparse<T, STRICT, COLL, true, true>);
-    }
-    if ((e = preload_kernel(k_step_sparse<T, STRICT, COLL, false, false>)) != cudaSuccess) return e;
-    return preload_kernel(k_step_sparse<T, STRICT, COLL, true, false>);
-}
-
 }  // namespace lbm

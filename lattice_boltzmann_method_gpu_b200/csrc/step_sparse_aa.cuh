@@ -330,102 +330,5 @@ __global__ void __launch_bounds__(PERSIST_BLOCK, sizeof(T) == 8 ? 1 : 2)
         if (s + 1 < pa.nsteps) grid_barrier(pa.barrier, (unsigned)(s + 1));
     }
 }
-template <typename T, bool STRICT, int COLL>
-cudaError_t launch_sparse_aa_persist_coll(const SparseParams<T> &p_in, const PersistArgs<T> &pa, int sm_count, cudaStream_t s) {
-    SparseParams<T> p = p_in;
-    for (int q = 0; q < Q; q++) {
-        p.base.pull_base[q] = p.base.src + (long long)q * p.base.qstride;
-        p.base.store_base[q] = p.base.dst + (long long)q * p.base.qstride;
-        p.dk[q] = (int)((long long)(q - oppq(q)) * p.base.qstride);
-    }
-    int per_sm = 0;
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sparse_aa_persist<T, STRICT, COLL>, PERSIST_BLOCK, 0);
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) return cudaErrorLaunchOutOfResources;
-    per_sm = std::min(per_sm, sizeof(T) == 8 ? 1 : 2);
-    const long long work = std::max((p.id_end - p.id_begin + 31) / 32 + 1, p.seg_end - p.seg_begin);
-    // as many warps as give every warp the same number of rounds (an uneven last round makes everybody wait)
-    const long long wpb = PERSIST_BLOCK / 32, max_blocks = std::min<long long>((long long)sm_count * per_sm, (long long)BAR_GROUP * 64);
-    const long long rounds = std::max<long long>(1, (work + max_blocks * wpb - 1) / (max_blocks * wpb));
-    const long long warps = (work + rounds - 1) / rounds;
-    long long blocks = std::max<long long>(1, std::min(max_blocks, (warps + wpb - 1) / wpb));
-    PersistArgs<T> a = pa;
-    void *args[2] = {(void *)&p, (void *)&a};
-    return cudaLaunchCooperativeKernel((const void *)k_sparse_aa_persist<T, STRICT, COLL>, dim3((unsigned)blocks), dim3(PERSIST_BLOCK), args, 0, s);
-}
-template <typename T, bool STRICT>
-cudaError_t launch_sparse_aa_persist_impl(const SparseParams<T> &p, const PersistArgs<T> &pa, int sm_count, cudaStream_t s) {
-    if (p.base.collision == LBM_COLL_BGK) return launch_sparse_aa_persist_coll<T, STRICT, LBM_COLL_BGK>(p, pa, sm_count, s);
-    if constexpr (!STRICT) {
-        if (p.base.collision == LBM_COLL_TRT) return launch_sparse_aa_persist_coll<T, false, LBM_COLL_TRT>(p, pa, sm_count, s);
-    }
-    return cudaErrorInvalidValue;
-}
-
-template <typename T, bool STRICT, int COLL, bool MOMENTS, bool RESID, bool PEERS>
-cudaError_t launch_sparse_aa_mode(const SparseParams<T> &p, cudaStream_t s) {
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cudaLaunchConfig_t cfg = {};
-    cfg.blockDim = dim3(SPARSE_BLOCK), cfg.dynamicSmemBytes = 0, cfg.stream = s;
-    cfg.attrs = at, cfg.numAttrs = (!PEERS && p.pdl) ? 1 : 0;
-    if (p.base.parity == 0) {
-        const long long n = p.id_end - p.id_begin;
-        if (n <= 0) return cudaSuccess;
-        cfg.gridDim = dim3((unsigned)((n + SPARSE_BLOCK - 1) / SPARSE_BLOCK));
-        return cudaLaunchKernelEx(&cfg, k_sparse_aa_even<T, STRICT, COLL, MOMENTS, RESID, PEERS>, p);
-    }
-    const long long nrec = p.seg_end - p.seg_begin;
-    if (nrec <= 0) return cudaSuccess;
-    const int wpb = SPARSE_BLOCK / 32;
-    cfg.gridDim = dim3((unsigned)((nrec + wpb - 1) / wpb));
-    return cudaLaunchKernelEx(&cfg, k_sparse_aa_odd<T, STRICT, COLL, MOMENTS, RESID, PEERS>, p);
-}
-
-template <typename T, bool STRICT, int COLL>
-cudaError_t launch_step_sparse_aa_coll(const SparseParams<T> &p_in, bool moments, bool resid, cudaStream_t s) {
-    SparseParams<T> p = p_in;
-    for (int q = 0; q < Q; q++) {
-        p.base.pull_base[q] = p.base.src + (long long)q * p.base.qstride;
-        p.base.store_base[q] = p.base.dst + (long long)q * p.base.qstride;
-        p.dk[q] = (int)((long long)(q - oppq(q)) * p.base.qstride);  // |q - opp q| <= 3, qstride < 2^31 / 3 (checked by the host)
-    }
-    const bool peers = p.base.peer_up || p.base.peer_dn;
-#define LBM_SPAA(M, R)                                                                    \
-    (peers ? launch_sparse_aa_mode<T, STRICT, COLL, M, R, true>(p, s) : launch_sparse_aa_mode<T, STRICT, COLL, M, R, false>(p, s))
-    if (moments && resid) return LBM_SPAA(true, true);
-    if (moments) return LBM_SPAA(true, false);
-    if (resid) return LBM_SPAA(false, true);
-    return LBM_SPAA(false, false);
-#undef LBM_SPAA
-}
-template <typename T, bool STRICT>
-cudaError_t launch_step_sparse_aa_impl(const SparseParams<T> &p, bool moments, bool resid, cudaStream_t s) {
-    if (p.base.collision == LBM_COLL_BGK) return launch_step_sparse_aa_coll<T, STRICT, LBM_COLL_BGK>(p, moments, resid, s);
-    if constexpr (!STRICT) {
-        if (p.base.collision == LBM_COLL_TRT) return launch_step_sparse_aa_coll<T, false, LBM_COLL_TRT>(p, moments, resid, s);
-    }
-    return cudaErrorInvalidValue;
-}
-
-template <typename T, bool STRICT, int COLL, bool PEERS>
-cudaError_t preload_sparse_aa_peers(bool resid) {
-    cudaError_t e;
-#define LBM_PL(M, R)                                                                                      \
-    if ((e = preload_kernel(k_sparse_aa_even<T, STRICT, COLL, M, R, PEERS>)) != cudaSuccess) return e;          \
-    if ((e = preload_kernel(k_sparse_aa_odd<T, STRICT, COLL, M, R, PEERS>)) != cudaSuccess) return e;
-    if (resid) {
-        LBM_PL(false, true) LBM_PL(true, true)
-    } else {
-        LBM_PL(false, false) LBM_PL(true, false)
-    }
-#undef LBM_PL
-    return cudaSuccess;
-}
-template <typename T, bool STRICT, int COLL>
-cudaError_t preload_step_sparse_aa_impl(bool peers, bool resid) {
-    return peers ? preload_sparse_aa_peers<T, STRICT, COLL, true>(resid) : preload_sparse_aa_peers<T, STRICT, COLL, false>(resid);
-}
 
 }  // namespace lbm

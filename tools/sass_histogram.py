@@ -12,11 +12,12 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parents[1]
 LIB = ROOT / "lattice_boltzmann_method_gpu_b200" / "liblbm_b200.so"
-WANT = ["k_step_dense<double, false, false, false, true, 2, 1>", "k_step_dense<double, false, false, false, true, 2, 2>",
-        "k_step_dense<float, false, false, false, true, 3, 1>", "k_step_dense<float, false, false, false, true, 3, 2>",
-        "k_sparse_aa_even<double, false, false, false, false>", "k_sparse_aa_odd<double, false, false, false, false>",
-        "k_sparse_aa_even<float, false, false, false, false>", "k_sparse_aa_odd<float, false, false, false, false>",
-        "k_step_sparse<double, false, false, false>", "k_sparse_aa_persist<float, false>"]
+# FAST arithmetic, BGK collision (COLL 0), no moments, no sum |u|; dense: speculative pull, in-place even / odd step
+WANT = ["k_step_dense<double, false, 0, false, false, true, 1>", "k_step_dense<double, false, 0, false, false, true, 2>",
+        "k_step_dense<float, false, 0, false, false, true, 1>", "k_step_dense<float, false, 0, false, false, true, 2>",
+        "k_sparse_aa_even<double, false, 0, false, false, false>", "k_sparse_aa_odd<double, false, 0, false, false, false>",
+        "k_sparse_aa_even<float, false, 0, false, false, false>", "k_sparse_aa_odd<float, false, 0, false, false, false>",
+        "k_step_sparse<double, false, 0, false, false>", "k_sparse_aa_persist<float, false, 0>"]
 GROUPS = [("LDG", r"^LDG"), ("STG", r"^STG"), ("LDL/STL (local)", r"^(LDL|STL)"), ("SHFL", r"^SHFL"), ("LDC/ULDC (constant bank)", r"^(LDC|ULDC|LDCU)"),
           ("integer (IADD3 IMAD LOP3 SHF LEA ISETP SEL VIADD ...)", r"^(IADD|IMAD|LOP3|SHF|LEA|ISETP|SEL|VIADD|IABS|MOV|PRMT|UIADD|UMOV|ULOP|USHF|UIMAD|R2P|P2R|PLOP|UISETP|ULEA|USEL)"),
           ("fp32 (FFMA FADD FMUL MUFU)", r"^(FFMA|FADD|FMUL|MUFU|FSETP|FSEL)"), ("fp64 (DFMA DADD DMUL)", r"^(DFMA|DADD|DMUL|DSETP)"),
