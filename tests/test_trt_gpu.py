@@ -35,50 +35,23 @@ def trt_case(name, n, prec, storage=None, magic=MAGIC, **kw):
     return c
 
 
-# bif runs with its inlet speeds halved (max 0.10): at the fixture's 0.21 (Mach 0.36) and tau = 0.55 the TRT run
-# diverges after ~150 steps, in the CPU reference as well -- a stability limit of that flow, not a difference
-BIF_INLET_SCALE = 0.5
-
-
-def parity_setup(c, name):
-    """geo_pre .. initialize of a GPU handle, with the inlet of parity_oracle"""
-    if name != "bif":
-        return H.gpu_setup(c, name)
-    c.geo_pre()
-    c.index_transform()
-    inl, out = H.bif_bc_planes()
-    c.set_bc_planes((inl * BIF_INLET_SCALE).astype(np.float32), out)
-    c.initialize()
-
-
-def parity_oracle(name, n, dt):
-    o, geo, *_ = H.oracle_case(name, n, dt)
-    if name == "bif":
-        inl, out = H.bif_bc_planes()
-        ny = geo.shape[1]
-        o.set_bc_planes(np.where(geo[:, 1, :] == 2, inl * BIF_INLET_SCALE, 0).astype(np.float32),
-                        np.where(geo[:, ny - 2, :] == 3, out, 0).astype(np.float32))
-        o.initialize()
-    return o
-
-
 @pytest.mark.parametrize("name,n", [("ldc", 32), ("pos", 24), ("bif", None), ("cor", None)])
 @pytest.mark.parametrize("prec,tol,steps,magic", [("f32", 1e-5, 100, MAGIC), ("f64", 1e-12, 400, MAGIC), ("f64", 1e-12, 400, 0.25)])
 def test_fast_trt_matches_trt_oracle(name, n, prec, tol, steps, magic):
     lib = L()
     dt = np.float32 if prec == "f32" else np.float64
     p = lib.F32 if prec == "f32" else lib.F64
-    o = parity_oracle(name, n, dt)
+    o, *_ = H.trt_oracle_case(name, n, dt)
     c = H.gpu_case(name, n, p, lib.MATH_FAST)
     c.set_collision(lib.COLL_TRT, magic)
-    parity_setup(c, name)
+    H.trt_gpu_setup(c, name)
     TRT.step(o, steps, magic)
     c.step(steps)
     err = H.rel_err(c.get_fields(), o.fields())
     assert err <= tol, f"{name} {prec} magic {magic}: rel err {err:.3e} > {tol}"
     # the operator is not BGK: the same run under BGK is far from the TRT reference
     b = H.gpu_case(name, n, p, lib.MATH_FAST)
-    parity_setup(b, name)
+    H.trt_gpu_setup(b, name)
     b.step(steps)
     assert H.rel_err(b.get_fields(), o.fields()) > 100 * tol
 
